@@ -24,6 +24,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -46,14 +47,14 @@ def host_cores():
 
 
 _CPU_THREADS = None
-CALIB_PATH = os.path.join(ROOT, ".kgx_cpu_calibration.json")
+CALIB_PATH = os.path.join(tempfile.gettempdir(), "kgx_cpu_calibration.json")   # the tree may be read-only
 
 
 def cpu_threads(be):
     """Thread count of the CPU arm, calibrated ONCE per box and shared by `--impl reference`, the cpu_baseline leg and the
     product-level run (VERDICT r1 weak #6: two calibrations in one driver run picked 64 and 32 threads).  The visible CPU
     count can exceed what the container may run (cgroup quota), so the candidate with the best short-run rate is kept and
-    cached on disk next to bench.py, keyed by host name and visible core count."""
+    cached in the temporary directory, keyed by host name and visible core count."""
     global _CPU_THREADS
     if _CPU_THREADS is not None:
         return _CPU_THREADS
@@ -228,7 +229,7 @@ def shim_prepare(eng, case, sc, local_rank):
     read back from the device, true distances mod n) -- called BEFORE any launch so that (x, y, d) are consistent."""
     import tempfile
     import numpy as np
-    if not os.path.exists(os.path.join(ROOT, "build", "kgx_shim_bench")):
+    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "kgx_shim_bench")):
         return None
     ax, ay, _ = eng.GetKangaroosRaw()
     tmp = tempfile.mkdtemp(prefix="kgx_shim_%d_" % local_rank)
@@ -243,12 +244,12 @@ def shim_prepare(eng, case, sc, local_rank):
 
 
 def shim_run(prep, gx, gy, local_rank, dp, warmup, steps):
-    """Headline e2e leg: K steps through the reference's C++ interface -- build/kgx_shim_bench constructs `class GPUEngine`
+    """Headline e2e leg: K steps through the reference's C++ interface -- oracle/_ref/kgx_shim_bench constructs `class GPUEngine`
     (reference header, GPUEngine_b200.cpp shim), SetKangaroos(Int*...) from host arrays, callKernel, K x Launch(std::vector<ITEM>&)
     with the per-record Int marshalling and ModSubK1order of the reference's Launch (GPUEngine.cu:653-675).
     -> (seconds for K steps, DP items returned, upload seconds)"""
     tmp, tab_path, herd_path = prep
-    exe = os.path.join(ROOT, "build", "kgx_shim_bench")
+    exe = os.path.join(ROOT, "oracle", "_ref", "kgx_shim_bench")
     try:
         p = subprocess.run([exe, str(local_rank), str(gx), str(gy), str(dp), str(warmup), str(steps), tab_path, herd_path],
                            capture_output=True, text=True, timeout=900)
@@ -270,6 +271,34 @@ def shim_run(prep, gx, gy, local_rank, dp, warmup, steps):
             pass
 
 
+def _words(a):
+    """(n, limbs) uint64 -> (n, 2*limbs) float64 of the 32-bit words, least significant first: exact in float64."""
+    import numpy as np
+    a = np.ascontiguousarray(a, dtype=np.uint64)
+    return np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).reshape(a.shape[0], -1).astype(np.float64)
+
+
+DUMP_KANGAROOS = 1 << 16
+
+
+def dump_outputs(eng, out_dir):
+    """What the timed path computed in its last launch, as a caller of the engine receives it: the DP records of that launch
+    (Launch(): x, distance mod n, kIdx; sorted by kIdx then x, since the device appends them in no fixed order) and the herd
+    state it left (GetKangaroos: x, y, biased device distance) for a fixed, seeded sample of DUMP_KANGAROOS kangaroos.  256-bit
+    values are split into 32-bit words (least significant first) so that float64 holds them exactly: about 11 MB in all."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(eng.Launch(relaunch=False), key=lambda it: (it.kIdx, it.x))
+    np.save(os.path.join(out_dir, "dp_x.npy"), _words(_limb_rows([it.x for it in items], 4)))
+    np.save(os.path.join(out_dir, "dp_d.npy"), _words(_limb_rows([it.d for it in items], 4)))
+    np.save(os.path.join(out_dir, "dp_kidx.npy"), np.array([it.kIdx for it in items], dtype=np.float64))
+    ax, ay, ad = eng.GetKangaroosRaw()
+    idx = np.sort(np.random.Generator(np.random.PCG64(2024)).choice(ax.shape[0], size=min(DUMP_KANGAROOS, ax.shape[0]), replace=False))
+    np.save(os.path.join(out_dir, "kangaroo_index.npy"), idx.astype(np.float64))
+    for name, a in (("kangaroo_x", ax), ("kangaroo_y", ay), ("kangaroo_d", ad)):
+        np.save(os.path.join(out_dir, name + ".npy"), _words(a[idx]))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -279,6 +308,8 @@ def main():
     ap.add_argument("--grid", default="", help="x,y override (default 2*SMs,128)")
     ap.add_argument("--dp", type=int, default=16)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed launch computed to DIR/*.npy (rank 0)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -377,6 +408,8 @@ def main():
     # the K timed launches are exactly the K kernels completed inside the region: (K-1) collected + the one synced
     kernel_ms = kernel_ms[1:] + [eng.last_launch_ms()]
     dev_s = sum(kernel_ms) / 1e3
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)
 
     # ---- end-to-end leg through the C ABI with HOST buffers: kgx_collect(..., relaunch=1) is exactly the body of
     # GPUEngine::Launch (GPUEngine.cu:607-679): wait for the kernel, start the next one, copy this launch's DP records
@@ -490,7 +523,7 @@ def main():
                          "how": "CUDA events on the engine stream around each jump_kernel launch"},
             e2e={"value": e2e_value, "unit": "MJump/s", "h2d_bytes_per_step": 0,
                  "d2h_bytes_per_step": (4 + shim_items * 56.0 / max(steps, 1)) if shim_s > 0 else d2h / max(steps, 1),
-                 "how": ("build/kgx_shim_bench: the reference's own `class GPUEngine` (unchanged header, GPUEngine_b200.cpp over libkgx.so): "
+                 "how": ("oracle/_ref/kgx_shim_bench: the reference's own `class GPUEngine` (unchanged header, GPUEngine_b200.cpp over libkgx.so): "
                          "SetKangaroos(Int*) once, then K x Launch(std::vector<ITEM>&) = wait, relaunch, DP records device -> host -> Int "
                          "marshalling + ModSubK1order per record (GPUEngine.cu:607-679); host-clock around the K calls, max over ranks"
                          if shim_s > 0 else

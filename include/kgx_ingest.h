@@ -4,11 +4,9 @@
  * What it replaces: the body of the DP loop of Kangaroo::SolveKeyGPU (reference Kangaroo.cpp:594-612: under ghMutex,
  * per DP `AddToTable` -> HashTable::Add (HashTable.cpp:221-307) -> on ADD_COLLISION `CollisionCheck`), and the server-side
  * drain of Thread.cpp:165-234, for the in-box multi-GPU case where the DP records of ALL ranks arrive on rank 0 as one
- * buffer per step (NCCL gather, kangaroo_b200/dist.py).  The table itself is the reference's own `class HashTable`,
- * UNCHANGED: this library is compiled against /root/reference (HashTable.cpp + SECPK1) exactly like the drop-in binary
- * (kangaroo_b200/csrc/build_ingest.sh); only the driver around it is new: records are inserted by a pool of worker threads
- * sharded by bucket index (h mod threads) -- buckets are independent in the reference's table, so no lock is needed --
- * instead of one thread under one mutex.
+ * buffer per step (NCCL gather, kangaroo_b200/dist.py).  The table keeps the semantics and the work-file layout of the
+ * reference's `class HashTable`; records are inserted by a pool of worker threads sharded by bucket index (h mod threads)
+ * -- buckets are independent, so no lock is needed -- instead of one thread under one mutex.
  *
  * Record format = the reference's wire/disk `DP` (Kangaroo.h:94-101), produced on the device by kgx_convert_dps():
  *   { uint32 kIdx; uint32 h; uint128 x (128 LSBs); uint128 d (b127 sign, b126 type, b125..0 |distance|) }   40 bytes.
@@ -52,7 +50,7 @@ int kgi_add(kgi_table* t, const void* dp40, uint32_t n, uint32_t rank, kgi_event
 int kgi_add_items(kgi_table* t, const void* items56, uint32_t n, uint32_t rank, const uint64_t wild_offset[2],
                   kgi_event* ev, uint32_t cap, uint32_t* n_ev);
 
-/* Kangaroo::CollisionCheck + CheckKey (Kangaroo.cpp:218-302) with the reference's own Secp256K1: given the two tagged
+/* Kangaroo::CollisionCheck + CheckKey (Kangaroo.cpp:218-302): given the two tagged
  * distances of a KGI_EV_COLLISION, the search key (keyToSearch = P - start*G, 4+4 limbs) and range start (4 limbs), writes
  * the private key (4 limbs) and returns 1 when one of the four sign combinations matches +-key, else 0. */
 int kgi_resolve(kgi_table* t, const uint64_t d_old[2], const uint64_t d_new[2], const uint64_t keyx[4], const uint64_t keyy[4],

@@ -8,6 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.environ.get("KGX_LIB_OVERRIDE") or os.path.join(CSRC, "libkgx.so")   # override: A/B builds in scripts/ experiments
 HOSTTEST_PATH = os.path.join(CSRC, "libkgx_hosttest.so")
+INGEST_PATH = os.path.join(CSRC, "libkgx_ingest.so")
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -60,13 +61,14 @@ _lib = None
 
 
 def build_library(verbose=False):
-    """Compile every CUDA source for sm_100a into csrc/libkgx.so (nvcc cross-compiles without a GPU) and the
-    host-only unit-test helper csrc/libkgx_hosttest.so."""
+    """Compile every CUDA source for sm_100a into csrc/libkgx.so (nvcc cross-compiles without a GPU), the rank-0 DP table
+    csrc/libkgx_ingest.so and the host-only unit-test helper csrc/libkgx_hosttest.so."""
     src = os.path.join(CSRC, "kgx_engine.cu")
     cmd = ["nvcc"] + NVCC_FLAGS + ["-o", LIB_PATH, src]
     if verbose:
         cmd += ["-Xptxas", "-v"]
     subprocess.check_call(cmd, cwd=CSRC)
+    subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-Wall", "-o", INGEST_PATH, os.path.join(CSRC, "kgx_ingest.cpp"), "-lpthread"])
     subprocess.check_call(["g++", "-O2", "-frounding-math", "-ffp-contract=off", "-fPIC", "-shared", "-o", HOSTTEST_PATH, os.path.join(CSRC, "kgx_hosttest.cpp")])
     return LIB_PATH
 

@@ -1,16 +1,15 @@
-"""ctypes binding of build/libkgx_ingest.so (C ABI: include/kgx_ingest.h): the rank-0 distinguished-point table.
+"""ctypes binding of csrc/libkgx_ingest.so (C ABI: include/kgx_ingest.h): the rank-0 distinguished-point table.
 
-The table is the reference's own `class HashTable` (HashTable.{h,cpp}, compiled unmodified from /root/reference by
-kangaroo_b200/csrc/build_ingest.sh); the library adds the batched, bucket-sharded multi-threaded insert that replaces the
-single-mutex loop of Kangaroo::SolveKeyGPU (Kangaroo.cpp:594-612) when the DP records of all GPUs arrive on rank 0.
+The table follows the reference's `class HashTable` (HashTable.{h,cpp}: same insert semantics, same work-file layout) and
+is filled by a batched, bucket-sharded multi-threaded insert that replaces the single-mutex loop of Kangaroo::SolveKeyGPU
+(Kangaroo.cpp:594-612) when the DP records of all GPUs arrive on rank 0.
 No Python-side fallback: without the library DPTable() raises."""
 import ctypes
 import os
 
 import numpy as np
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.path.join(HERE, "..", "build", "libkgx_ingest.so")
+from ._lib import INGEST_PATH as LIB_PATH
 
 EV_RESET, EV_COLLISION = 1, 2
 DP40_BYTES, ITEM_BYTES = 40, 56
@@ -50,7 +49,7 @@ def load_library():
         return _lib
     path = os.path.abspath(LIB_PATH)
     if not os.path.exists(path):
-        raise RuntimeError("kangaroo_b200: %s is missing (kangaroo_b200/csrc/build_ingest.sh builds it against the reference sources)" % path)
+        raise RuntimeError("kangaroo_b200: %s is missing (run __graft_entry__.build())" % path)
     lib = ctypes.CDLL(path)
     for name, (res, args) in _SIGS.items():
         fn = getattr(lib, name)
@@ -64,7 +63,7 @@ def _limbs4(v):
 
 
 class DPTable:
-    """Rank-0 DP table: reference HashTable + sharded batched insert (Kangaroo::AddToTable semantics per record)."""
+    """Rank-0 DP table: HashTable semantics + sharded batched insert (Kangaroo::AddToTable semantics per record)."""
 
     def __init__(self, threads=0, max_events=4096):
         self._lib = load_library()
@@ -125,7 +124,7 @@ class DPTable:
         return self._events(ne.value)
 
     def resolve(self, d_old, d_new, key, range_start):
-        """Kangaroo::CollisionCheck/CheckKey with the reference's Secp256K1 -> private key (int) or None."""
+        """Kangaroo::CollisionCheck/CheckKey -> private key (int) or None."""
         a = (ctypes.c_uint64 * 2)(*d_old); b = (ctypes.c_uint64 * 2)(*d_new)
         out = (ctypes.c_uint64 * 4)()
         rc = self._lib.kgi_resolve(self._h, a, b, _limbs4(key[0]), _limbs4(key[1]), _limbs4(range_start), out)

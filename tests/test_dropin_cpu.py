@@ -7,13 +7,13 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BIN = os.path.join(ROOT, "build", "kangaroo_b200")
+BIN = os.path.join(ROOT, "oracle", "_ref", "kangaroo_b200")
 EXPECTED = ["57004A31CED094F0", "57004A31D2F397AF", "57004A00A71C8425", "57004A73420E46DF", "57004ACEF20EBCFD"]
 
 
 def test_in40_cpu_only_through_dropin_binary():
     if not os.path.exists(BIN):
-        pytest.skip("build/kangaroo_b200 not built (needs the reference sources at build time)")
+        pytest.skip("oracle/_ref/kangaroo_b200 not built (needs the reference sources at build time)")
     p = subprocess.run([BIN, "-t", "2", os.path.join(ROOT, "tests", "golden", "in40_5.txt")], capture_output=True, text=True,
                        timeout=600, cwd=ROOT)
     out = (p.stdout + p.stderr).upper()

@@ -1,5 +1,5 @@
 """-m gpu: the reference's UNMODIFIED host program (main/Kangaroo/Check/HashTable/SECPK1, compiled from
-/root/reference by kangaroo_b200/csrc/build_dropin.sh) linked against the B200 engine through the GPUEngine shim.
+the reference sources by oracle/build_dropin.sh) linked against the B200 engine through the GPUEngine shim.
   * `-check`  = the reference's own parity test, Check.cpp:467-621 (GPU vs CPU after NB_RUN jumps + DP set)
   * in56 / in64 = end-to-end solves with published answers (README.md:146-147, 194-195)
 The binary is built in the build container (the reference sources do not exist on the GPU box) and travels."""
@@ -10,13 +10,13 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BIN = os.path.join(ROOT, "build", "kangaroo_b200")
+BIN = os.path.join(ROOT, "oracle", "_ref", "kangaroo_b200")
 GOLD = os.path.join(ROOT, "tests", "golden")
 
 
 def run(args, timeout=600, env=None):
     if not os.path.exists(BIN):
-        pytest.skip("build/kangaroo_b200 not built (needs the reference sources at build time)")
+        pytest.skip("oracle/_ref/kangaroo_b200 not built (needs the reference sources at build time)")
     e = dict(os.environ)
     e.update(env or {})
     p = subprocess.run([BIN] + args, capture_output=True, text=True, timeout=timeout, cwd=ROOT, env=e)

@@ -7,7 +7,7 @@ The reference has two symmetric jump rules behind its compile-time switch; the e
 Both: P += J, d += jD mod n, class switch (y > (p-1)/2 -> y = p - y, d = n - d).  Restated in oracle/kgx_oracle.c
 (kgo_jump_sym), pinned to the reference's Int / IntGroup code by tests/test_oracle_vs_ref.py.  Checked here
   * through the C ABI on every jump kernel (state + DP multiset, several launches so lastJump persists across launches),
-  * through the reference's UNMODIFIED host compiled with -DUSE_SYMMETRY and linked to the engine (build/kangaroo_b200_sym):
+  * through the reference's UNMODIFIED host compiled with -DUSE_SYMMETRY and linked to the engine (oracle/_ref/kangaroo_b200_sym):
     its own `-check` prints CPU/GPU ok (KGX_SYM_RULE=lastjump) -- which the reference's own symmetric GPU kernel cannot
     (DESIGN.md, symmetry) -- and in64 is solved with the default symclass rule,
   * statistically: operations per solved key with and without symmetry (the reference's -DSTATS counters), ~1/sqrt(2)."""
@@ -148,9 +148,9 @@ def test_symmetric_device_hash_convert(oracle, kernel):
 
 
 def run(binary, args, timeout=900, env=None, cwd=None):
-    exe = os.path.join(ROOT, "build", binary)
+    exe = os.path.join(ROOT, "oracle", "_ref", binary)
     if not os.path.exists(exe):
-        pytest.skip("build/%s not built (needs the reference sources at build time)" % binary)
+        pytest.skip("oracle/_ref/%s not built (needs the reference sources at build time)" % binary)
     e = dict(os.environ); e.update(env or {})
     p = subprocess.run([exe] + args, capture_output=True, text=True, timeout=timeout, cwd=cwd or ROOT, env=e)
     return (p.stdout + p.stderr).replace("\r", "\n")
@@ -194,8 +194,7 @@ def test_symmetry_gain_in_operations_per_key(tmp_path):
     # involved) gives 2.30 vs 2.17 sqrt(N) over 96 keys of a 2^44 range (ratio 0.95, 25 dead kangaroos per key instead of 1.6).
     # So this is a record + sanity bound (64-key averages scatter by ~9 %), not a claim of the theoretical gain.
     assert sym < 1.25 * plain, avgs
-    os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-    with open(os.path.join(ROOT, "gpurun_out", "symmetry_gain.txt"), "w") as f:
+    with open(str(tmp_path / "symmetry_gain.txt"), "w") as f:
         f.write("64 keys, 2^56 range, grid 4x128 (65,536 kangaroos), dp 9, reference host (-DSTATS) + B200 engine\n")
         f.write("plain    : %.3f sqrt(N) operations per key (reference's estimate %.3f)\n" % avgs["kangaroo_b200_stats"])
         f.write("symmetry : %.3f sqrt(N) operations per key (reference's estimate %.3f)\n" % avgs["kangaroo_b200_sym_stats"])

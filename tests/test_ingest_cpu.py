@@ -1,21 +1,22 @@
-"""CPU: the rank-0 DP ingest (build/libkgx_ingest.so = kgx_ingest.cpp + the reference's unmodified HashTable/SECPK1).
-Semantics pinned to Kangaroo::AddToTable / CollisionCheck / CheckKey (Kangaroo.cpp:218-330) and to the reference's own work-file
-checker (`kangaroo -wcheck`, Check.cpp:33-108,290-411) run on a file written by kgi_save_work."""
+"""CPU: the rank-0 DP ingest (kangaroo_b200/csrc/libkgx_ingest.so = kgx_ingest.cpp).
+Semantics pinned to Kangaroo::AddToTable / CollisionCheck / CheckKey (Kangaroo.cpp:218-330), and the work file written by
+kgi_save_work to the one the reference's HashTable writes for the same records (tests/golden/work_file_golden.json), plus the
+reference's own work-file checker (`kangaroo -wcheck`, Check.cpp:33-108,290-411) where oracle/_ref is built."""
+import hashlib
+import json
 import os
 import struct
 import subprocess
 import time
 
 import numpy as np
-import pytest
 
 from kangaroo_b200 import ecmath as ec
+from kangaroo_b200.ingest import LIB_PATH as INGEST
 from oracle import kgo
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-INGEST = os.path.join(ROOT, "build", "libkgx_ingest.so")
 REFBIN = os.path.join(ROOT, "oracle", "_ref", "kangaroo_ref_cpu")
-pytestmark = pytest.mark.skipif(not os.path.exists(INGEST), reason="build/libkgx_ingest.so not built (needs the reference sources at build time)")
 
 M64 = (1 << 64) - 1
 
@@ -113,10 +114,11 @@ def test_collision_resolves_to_the_key(oracle):
     t.close()
 
 
-@pytest.mark.skipif(not os.path.exists(REFBIN), reason="oracle/_ref/kangaroo_ref_cpu not built")
 def test_work_file_passes_the_reference_wcheck(oracle, tmp_path):
-    """f3 format half: DPs of a real walk -> kgi_add_items -> kgi_save_work; the reference's own `-winfo` reads the header and
-    `-wcheck` recomputes d*G (+P) for every stored DP and compares x and the bucket (Check.cpp:33-108)."""
+    """f3 format half: DPs of a real walk -> kgi_add_items -> kgi_save_work.  The file must be byte for byte the one the
+    reference's HashTable::SaveTable writes for the same records (tests/golden/work_file_golden.json);
+    where the reference build exists, its own `-winfo` reads the header and `-wcheck` recomputes d*G (+P) for every stored DP
+    and compares x and the bucket (Check.cpp:33-108)."""
     from kangaroo_b200.ingest import DPTable
     rp = 64
     start = 0x5B3F38AF935A3640D158E871CE6E9666DB862636383386EE0000000000000000
@@ -140,10 +142,15 @@ def test_work_file_passes_the_reference_wcheck(oracle, tmp_path):
     assert n > 4000
     path = str(tmp_path / "kgx.work")
     t.save_work(path, 6, start, end, pub, total_count=2048 * 256, total_time=1.5)
-    out = subprocess.run([REFBIN, "-winfo", path], capture_output=True, text=True, timeout=120).stdout
-    assert str(n) in out and "DP" in out, out
-    out = subprocess.run([REFBIN, "-wcheck", path], capture_output=True, text=True, timeout=300).stdout
-    assert "[100.000% OK]" in out and "Wrong" not in out, out[-1500:]      # Check.cpp:393-409
+    golden = json.load(open(os.path.join(ROOT, "tests", "golden", "work_file_golden.json")))
+    data = open(path, "rb").read()
+    assert (n, len(data)) == (golden["dp_count"], golden["bytes"])
+    assert hashlib.sha256(data).hexdigest() == golden["sha256"]
+    if os.path.exists(REFBIN):
+        out = subprocess.run([REFBIN, "-winfo", path], capture_output=True, text=True, timeout=120).stdout
+        assert str(n) in out and "DP" in out, out
+        out = subprocess.run([REFBIN, "-wcheck", path], capture_output=True, text=True, timeout=300).stdout
+        assert "[100.000% OK]" in out and "Wrong" not in out, out[-1500:]  # Check.cpp:393-409
     # and the file loads back into an identical table
     t2 = DPTable(threads=2, max_events=1 << 16)
     assert t2.load_work(path)[0] == 6 and len(t2) == n
