@@ -91,6 +91,29 @@ int kgx_patch(kgx_engine* e, uint64_t kidx, const uint64_t px[4], const uint64_t
 int kgx_snapshot_begin(kgx_engine* e);
 int kgx_snapshot_read(kgx_engine* e, uint64_t* px, uint64_t* py, uint64_t* d);
 
+/* --- work-file walks (reference: Kangaroo::SaveWork with -ws, Backup.cpp:535-545; FetchWalks, Backup.cpp:211-231).
+ *     One KGX_WALK_SIZE-byte record per kangaroo, record i = kIdx i (herd type = i & 1): {x[4], y[4], d[4]} as 64-bit
+ *     little-endian limbs, d the UNBIASED distance mod n (wild: biased - wild_offset mod n; symmetric engines: the signed
+ *     distance mod n, wild_offset ignored) -- what GetKangaroos returns.
+ *   kgx_walks_begin  converts the herd into device staging in stream order (after the launch in flight) and returns
+ *                    without blocking the caller or later launches;
+ *   kgx_walks_read   waits for that conversion only and copies records [first, first + count) to `out` on a stream of
+ *                    its own (pinned `out` makes it fast); may be called from another host thread than the launches;
+ *   kgx_walks_end    ends the export (waits for the conversion if it is still running); the n x 96-byte staging
+ *                    buffer is kept for the next export and freed by kgx_destroy;
+ *   kgx_walks_load   writes `count` <= n records to kIdx [0, count) (distances re-biased and truncated to 128 bits like
+ *                    SetKangaroos; padding slots follow; lastJump / symClass reset), leaving the other kangaroos as they
+ *                    are.  verify != 0: recomputes d*G (tame) / key + d*G (wild; +-key on symmetric engines) for every
+ *                    record, *n_bad = records that do not match, their first bad_cap indices (ascending) in bad_idx.
+ *     Refused while a snapshot or a walk export is pending. --- */
+#define KGX_WALK_SIZE 96
+int kgx_walks_begin(kgx_engine* e, const uint64_t wild_offset[2]);
+int kgx_walks_read(kgx_engine* e, void* out, uint64_t first, uint64_t count);
+int kgx_walks_end(kgx_engine* e);
+int kgx_walks_load(kgx_engine* e, const void* recs, uint64_t count, const uint64_t wild_offset[2],
+                   const uint64_t keyx[4], const uint64_t keyy[4], int verify,
+                   uint64_t* n_bad, uint64_t* bad_idx, uint32_t bad_cap);
+
 /* --- herd creation on the device (SURVEY 8f/f2; replaces the CPU side of Kangaroo::CreateHerd, Kangaroo.cpp:670-738):
  *     kangaroo i starts at scalars[i]*G, plus `key` when (i + first_type) is odd (wild).  scalars: n x 4 limbs (mod the
  *     group order), d128: n x 2 limbs stored as the (biased) distances. --- */

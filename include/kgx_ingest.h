@@ -63,6 +63,22 @@ int kgi_save_work(kgi_table* t, const char* path, uint32_t dp_bits, const uint64
 /* Load the DP table of a reference work file (HEADW) into t; fills dp_bits / count / time when non-NULL.  0 on success. */
 int kgi_load_work(kgi_table* t, const char* path, uint32_t* dp_bits, uint64_t* total_count, double* total_time);
 
+/* Work file with kangaroos (the reference's -ws, Backup.cpp:530-547): the same bytes as kgi_save_work except that the
+ * trailing walk count is total_walks, and the file is extended (ftruncate) to its final length
+ *   *walk_offset + total_walks * KGI_WALK_SIZE,   *walk_offset = 156 + 2^18 * 8 + 32 * entries + 8
+ * so that the walk records can then be written in place -- by several processes, each pwrite-ing its own slice. */
+#define KGI_WALK_SIZE 96
+int kgi_save_work_walks(kgi_table* t, const char* path, uint32_t dp_bits, const uint64_t range_start[4], const uint64_t range_end[4],
+                        const uint64_t keyx[4], const uint64_t keyy[4], uint64_t total_count, double total_time,
+                        uint64_t total_walks, uint64_t* walk_offset);
+/* kgi_load_work plus everything else in the header: range start / end and key (4 limbs each), the walk count and the byte
+ * offset of the first walk record.  t may be NULL: the table is then skipped, not loaded.  Any output may be NULL.
+ * Returns 0, -1 when the file is not a readable HEADW work file, -2 when its key does not lie on the curve
+ * (Backup.cpp:175-179). */
+int kgi_load_work_ex(kgi_table* t, const char* path, uint32_t* dp_bits, uint64_t range_start[4], uint64_t range_end[4],
+                     uint64_t keyx[4], uint64_t keyy[4], uint64_t* total_count, double* total_time,
+                     uint64_t* n_walks, uint64_t* walk_offset);
+
 #ifdef __cplusplus
 }
 #endif

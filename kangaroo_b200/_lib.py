@@ -40,6 +40,11 @@ _SIGS = {
     "kgx_create_herd": (ctypes.c_int, [ctypes.c_void_p, _u64p, _u64p, _u64p, _u64p, ctypes.c_int]),
     "kgx_snapshot_begin": (ctypes.c_int, [ctypes.c_void_p]),
     "kgx_snapshot_read": (ctypes.c_int, [ctypes.c_void_p, _u64p, _u64p, _u64p]),
+    "kgx_walks_begin": (ctypes.c_int, [ctypes.c_void_p, _u64p]),
+    "kgx_walks_read": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64]),
+    "kgx_walks_end": (ctypes.c_int, [ctypes.c_void_p]),
+    "kgx_walks_load": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, _u64p, _u64p, _u64p, ctypes.c_int,
+                                      _u64p, _u64p, ctypes.c_uint32]),
     "kgx_launch_async": (ctypes.c_int, [ctypes.c_void_p]),
     "kgx_collect": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(Item), ctypes.c_uint32, ctypes.POINTER(ctypes.c_uint32),
                                    ctypes.POINTER(ctypes.c_uint32), ctypes.c_int, ctypes.c_int]),

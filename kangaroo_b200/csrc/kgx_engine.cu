@@ -13,6 +13,7 @@
 #include "../../include/kgx.h"
 #include "kgx_kernel.cuh"
 #include "kgx_herd.cuh"
+#include "kgx_walks.cuh"
 
 using namespace kgx;
 
@@ -49,6 +50,10 @@ struct kgx_engine {
   cudaEvent_t evStart[2] = {nullptr, nullptr}, evStop[2] = {nullptr, nullptr};
   cudaEvent_t evSnap = nullptr;   // snapshot (checkpoint) staging complete
   bool snapPending = false;
+  u64* stgW = nullptr;            // walk export staging: n x 96-byte work-file records (allocated by the first kgx_walks_begin)
+  cudaStream_t walkStream = nullptr;   // D2H of exported walks: its own stream, so kgx_collect's copies never queue behind it
+  cudaEvent_t evWalks = nullptr;  // walk export complete
+  bool walksPending = false;
   float lastMs = 0.f;
   unsigned long long* prof = nullptr;   // KGX_PROF=1: phase cycle counters
   u64 launches = 0;
@@ -120,6 +125,9 @@ void kgx_destroy(kgx_engine* e) {
   if (e->slabPinned) cudaFreeHost(e->slabPinned);
   for (int i = 0; i < 2; i++) { if (e->evStart[i]) cudaEventDestroy(e->evStart[i]); if (e->evStop[i]) cudaEventDestroy(e->evStop[i]); }
   if (e->evSnap) cudaEventDestroy(e->evSnap);
+  cudaFree(e->stgW);
+  if (e->evWalks) cudaEventDestroy(e->evWalks);
+  if (e->walkStream) cudaStreamDestroy(e->walkStream);
   if (e->stream) cudaStreamDestroy(e->stream);
   if (e->copyStream) cudaStreamDestroy(e->copyStream);
   delete e;
@@ -380,6 +388,96 @@ int kgx_snapshot_read(kgx_engine* e, uint64_t* px, uint64_t* py, uint64_t* d) {
   e->snapPending = false;
   free_staging(e);
   return 0;
+}
+
+// ---- work-file walks (kgx_walks.cuh; reference: SaveWork -ws, Backup.cpp:535-545, FetchWalks :211-231) ----
+// kgx_walks_begin converts the herd into 96-byte records in device staging, enqueued in stream order (after the launch
+// in flight) like kgx_snapshot_begin, and returns at once.  kgx_walks_read copies a range of them out on the walk stream
+// and waits for that copy only, so a writer thread can drain the export while the caller keeps launching.
+int kgx_walks_begin(kgx_engine* e, const uint64_t wild_offset[2]) {
+  CK(e, cudaSetDevice(e->dev));
+  if (e->walksPending) { snprintf(e->err, sizeof e->err, "kgx_walks_begin: previous walk export not ended"); return -1; }
+  if (e->snapPending) { snprintf(e->err, sizeof e->err, "kgx_walks_begin: snapshot pending (read it first)"); return -1; }
+  if (!e->stgW) CK(e, cudaMalloc(&e->stgW, (size_t)e->n * KGX_WALK_SIZE));
+  if (!e->walkStream) CK(e, cudaStreamCreateWithFlags(&e->walkStream, cudaStreamNonBlocking));
+  if (!e->evWalks) CK(e, cudaEventCreateWithFlags(&e->evWalks, cudaEventBlockingSync | cudaEventDisableTiming));
+  walks_export_kernel<<<(u32)((e->n + 255) / 256), 256, 0, e->stream>>>(e->state, e->stgW, e->n, e->T, e->K,
+                                                                         wild_offset[0], wild_offset[1], e->symmetry ? 1 : 0);
+  e->launches++;
+  CK(e, cudaGetLastError());
+  CK(e, cudaEventRecord(e->evWalks, e->stream));
+  e->walksPending = true;
+  return 0;
+}
+
+int kgx_walks_read(kgx_engine* e, void* out, uint64_t first, uint64_t count) {
+  CK(e, cudaSetDevice(e->dev));
+  if (!e->walksPending) { snprintf(e->err, sizeof e->err, "kgx_walks_read: no walk export pending"); return -1; }
+  if (first > e->n || count > e->n - first) { snprintf(e->err, sizeof e->err, "kgx_walks_read: range past the herd"); return -1; }
+  if (count == 0) return 0;
+  CK(e, cudaStreamWaitEvent(e->walkStream, e->evWalks, 0));
+  CK(e, cudaMemcpyAsync(out, e->stgW + first * WALK_WORDS, (size_t)count * KGX_WALK_SIZE, cudaMemcpyDeviceToHost, e->walkStream));
+  CK(e, cudaStreamSynchronize(e->walkStream));
+  return 0;
+}
+
+int kgx_walks_end(kgx_engine* e) {
+  CK(e, cudaSetDevice(e->dev));
+  if (!e->walksPending) return 0;
+  CK(e, cudaEventSynchronize(e->evWalks));
+  e->walksPending = false;   // stgW stays allocated for the next export (freed by kgx_destroy): no cudaMalloc / cudaFree,
+                             // which can block or synchronise the device, on every checkpoint
+  return 0;
+}
+
+int kgx_walks_load(kgx_engine* e, const void* recs, uint64_t count, const uint64_t wild_offset[2],
+                   const uint64_t keyx[4], const uint64_t keyy[4], int verify,
+                   uint64_t* n_bad, uint64_t* bad_idx, uint32_t bad_cap) {
+  CK(e, cudaSetDevice(e->dev));
+  if (e->walksPending || e->snapPending) { snprintf(e->err, sizeof e->err, "kgx_walks_load: snapshot or walk export pending"); return -1; }
+  if (count > e->n) { snprintf(e->err, sizeof e->err, "kgx_walks_load: %llu records for a herd of %llu", (unsigned long long)count, (unsigned long long)e->n); return -1; }
+  if (n_bad) *n_bad = 0;
+  if (count == 0) return 0;
+  if (verify && !e->herdTab) {
+    CK(e, cudaMalloc(&e->herdTab, 256 * 16 * 4));
+    herd_table_kernel<<<1, 32, 0, e->stream>>>(e->herdTab);
+    e->launches++;
+    CK(e, cudaGetLastError());
+  }
+  u64* dRecs = nullptr; u32* dKey = nullptr; uint8_t* dBad = nullptr;
+  uint8_t* hBad = nullptr;
+  uint64_t key[8];
+  memcpy(key, keyx, 32); memcpy(key + 4, keyy, 32);
+  auto body = [&]() -> int {      // CK returns from the lambda, so the scratch buffers are always released below
+    CK(e, cudaMalloc(&dRecs, (size_t)count * KGX_WALK_SIZE));
+    CK(e, cudaMemcpyAsync(dRecs, recs, (size_t)count * KGX_WALK_SIZE, cudaMemcpyHostToDevice, e->stream));
+    walks_import_kernel<<<(u32)((e->nPadded + 255) / 256), 256, 0, e->stream>>>(e->state, dRecs, count, e->n, e->nPadded, e->T, e->K,
+        wild_offset[0], wild_offset[1], e->symmetry ? 1 : 0, e->aux, e->symRule == KGX_SYM_CLASS ? 0 : 32);
+    e->launches++;
+    CK(e, cudaGetLastError());
+    if (verify) {
+      CK(e, cudaMalloc(&dKey, 64));
+      CK(e, cudaMalloc(&dBad, count));
+      CK(e, cudaMemcpyAsync(dKey, key, 64, cudaMemcpyHostToDevice, e->stream));
+      walks_verify_kernel<<<(u32)((count + 127) / 128), 128, 0, e->stream>>>(e->herdTab, dRecs, count, dKey, e->symmetry ? 1 : 0, dBad);
+      e->launches++;
+      CK(e, cudaGetLastError());
+      hBad = static_cast<uint8_t*>(malloc(count));
+      if (!hBad) { snprintf(e->err, sizeof e->err, "kgx_walks_load: out of host memory"); return -1; }
+      CK(e, cudaMemcpyAsync(hBad, dBad, count, cudaMemcpyDeviceToHost, e->stream));
+    }
+    CK(e, cudaStreamSynchronize(e->stream));
+    if (verify) {
+      uint64_t nb = 0;
+      for (uint64_t i = 0; i < count; i++)
+        if (hBad[i]) { if (bad_idx && nb < bad_cap) bad_idx[nb] = i; nb++; }
+      if (n_bad) *n_bad = nb;
+    }
+    return 0;
+  };
+  const int rc = body();
+  cudaFree(dRecs); cudaFree(dKey); cudaFree(dBad); free(hBad);
+  return rc;
 }
 
 int kgx_patch(kgx_engine* e, uint64_t kidx, const uint64_t px[4], const uint64_t py[4], const uint64_t d[2]) {

@@ -48,21 +48,12 @@ __global__ void herd_table_kernel(u32* tab) {
   }
 }
 
-// One thread per kangaroo: (x,y) = d*G [+ key].  scal: n x 8 words (d mod group order), key: 16 words or NULL rows
-// where isWild[i]==0.  Writes AoS px,py (n x 8 words each) in kIdx order.
-// sym != 0 (USE_SYMMETRY herd, Kangaroo.cpp:730-734): a point whose y is in the upper half is replaced by its negative and
-// the stored (signed 128-bit) distance dist[i] is negated with it.
-__global__ void herd_kernel(const u32* __restrict__ tab, const u32* __restrict__ scal, const u32* __restrict__ key,
-                            int firstType, u64 n, u32* px, u32* py, int sym, u32* dist) {
-  u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  u32 k[8];
-#pragma unroll
-  for (int w = 0; w < 8; w++) k[w] = scal[i * 8 + w];
-  u32 X[8], Y[8], Z[8];
+// (X, Y) = k*G [+ key] in canonical affine form (key: 16 words x then y, NULL for none).  Returns false for the point
+// at infinity (X, Y untouched).  Shared by herd creation and the work-file walk check (kgx_walks.cuh).
+__device__ __forceinline__ bool herd_point(const u32* __restrict__ tab, const u32* k, const u32* key, u32* X, u32* Y) {
+  u32 Z[8];
   bool inf = true;
-  const bool wild = ((i + (u64)firstType) & 1ull) != 0;
-  const int nterms = 256 + (wild ? 1 : 0);
+  const int nterms = 256 + (key ? 1 : 0);
   for (int b = 0; b < nterms; b++) {
     const u32* q;
     if (b < 256) {
@@ -116,14 +107,7 @@ __global__ void herd_kernel(const u32* __restrict__ tab, const u32* __restrict__
     fe_mul(Z, Z, h);                             // Z3
     fe_copy(X, t);
   }
-  if (inf) {
-    // scalar 0 (tame) or d*G == -key (wild): the point at infinity has no affine form; store (0, 0) -- not on the curve,
-    // the walk from it is meaningless but harmless (probability ~2^-rangePower; the reference stores an equally
-    // meaningless Z = 0 projective conversion, SECP256K1.cpp:59-87).
-#pragma unroll
-    for (int w = 0; w < 8; w++) { px[i * 8 + w] = 0; py[i * 8 + w] = 0; }
-    return;
-  }
+  if (inf) return false;
   u32 zi[8], zi2[8];
   modinv256(zi, Z);
   fe_sqr(zi2, zi);
@@ -142,6 +126,30 @@ __global__ void herd_kernel(const u32* __restrict__ tab, const u32* __restrict__
       acc = (u64)V[1] + 1u + (acc >> 32); V[1] = (u32)acc;
       for (int w = 2; w < 8; w++) { acc = (u64)V[w] + (acc >> 32); V[w] = (u32)acc; }
     }
+  }
+  return true;
+}
+
+// One thread per kangaroo: (x,y) = d*G [+ key].  scal: n x 8 words (d mod group order), key: 16 words or NULL rows
+// where isWild[i]==0.  Writes AoS px,py (n x 8 words each) in kIdx order.
+// sym != 0 (USE_SYMMETRY herd, Kangaroo.cpp:730-734): a point whose y is in the upper half is replaced by its negative and
+// the stored (signed 128-bit) distance dist[i] is negated with it.
+__global__ void herd_kernel(const u32* __restrict__ tab, const u32* __restrict__ scal, const u32* __restrict__ key,
+                            int firstType, u64 n, u32* px, u32* py, int sym, u32* dist) {
+  u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  u32 k[8];
+#pragma unroll
+  for (int w = 0; w < 8; w++) k[w] = scal[i * 8 + w];
+  u32 X[8], Y[8];
+  const bool wild = ((i + (u64)firstType) & 1ull) != 0;
+  if (!herd_point(tab, k, wild ? key : nullptr, X, Y)) {
+    // scalar 0 (tame) or d*G == -key (wild): the point at infinity has no affine form; store (0, 0) -- not on the curve,
+    // the walk from it is meaningless but harmless (probability ~2^-rangePower; the reference stores an equally
+    // meaningless Z = 0 projective conversion, SECP256K1.cpp:59-87).
+#pragma unroll
+    for (int w = 0; w < 8; w++) { px[i * 8 + w] = 0; py[i * 8 + w] = 0; }
+    return;
   }
   if (sym) {
     const u32 neg = fe_gt_half_mask(Y);

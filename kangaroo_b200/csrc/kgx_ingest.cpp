@@ -20,6 +20,8 @@
 #include <mutex>
 #include <thread>
 #include <vector>
+#include <sys/types.h>
+#include <unistd.h>
 #include "../../include/kgx_ingest.h"
 
 #define HEADW_MAGIC 0xFA6A8001u      // Kangaroo.h:120
@@ -351,24 +353,47 @@ int kgi_resolve(kgi_table* t, const uint64_t d_old[2], const uint64_t d_new[2], 
   return 0;
 }
 
-int kgi_save_work(kgi_table* t, const char* path, uint32_t dp_bits, const uint64_t range_start[4], const uint64_t range_end[4],
-                  const uint64_t keyx[4], const uint64_t keyy[4], uint64_t total_count, double total_time) {
-  FILE* f = fopen(path, "wb");
-  if (!f) return -1;
-  // Kangaroo::SaveHeader (Backup.cpp:368-394), type HEADW, then HashTable::SaveTable (HashTable.cpp:375-396)
+// Kangaroo::SaveHeader (Backup.cpp:368-394), type HEADW, then HashTable::SaveTable (HashTable.cpp:375-396) and the walk
+// count (Backup.cpp:530-551).  Returns the byte offset just past the walk count (the first walk record), or -1.
+static long long write_work(kgi_table* t, FILE* f, uint32_t dp_bits, const uint64_t range_start[4], const uint64_t range_end[4],
+                            const uint64_t keyx[4], const uint64_t keyy[4], uint64_t total_count, double total_time, uint64_t total_walks) {
   const uint32_t head = HEADW_MAGIC, version = 0;
   bool ok = fwrite(&head, 4, 1, f) == 1 && fwrite(&version, 4, 1, f) == 1 && fwrite(&dp_bits, 4, 1, f) == 1;
   ok = ok && fwrite(range_start, 32, 1, f) == 1 && fwrite(range_end, 32, 1, f) == 1;
   ok = ok && fwrite(keyx, 32, 1, f) == 1 && fwrite(keyy, 32, 1, f) == 1;
   ok = ok && fwrite(&total_count, 8, 1, f) == 1 && fwrite(&total_time, 8, 1, f) == 1;
+  long long pos = 156;
   for (uint32_t h = 0; ok && h < HASH_SIZE; h++) {
     const Bucket& b = t->buckets[h];
     const uint32_t nb = (uint32_t)b.items.size();
     ok = fwrite(&nb, 4, 1, f) == 1 && fwrite(&b.cap, 4, 1, f) == 1 && fwrite(b.items.data(), sizeof(Entry), nb, f) == nb;
+    pos += 8 + (long long)sizeof(Entry) * nb;
   }
-  const uint64_t totalWalk = 0;                                   // no kangaroos in this file (Backup.cpp:549-551)
-  ok = ok && fwrite(&totalWalk, 8, 1, f) == 1;
+  ok = ok && fwrite(&total_walks, 8, 1, f) == 1;
+  return ok ? pos + 8 : -1;
+}
+
+int kgi_save_work(kgi_table* t, const char* path, uint32_t dp_bits, const uint64_t range_start[4], const uint64_t range_end[4],
+                  const uint64_t keyx[4], const uint64_t keyy[4], uint64_t total_count, double total_time) {
+  FILE* f = fopen(path, "wb");
+  if (!f) return -1;
+  // no kangaroos in this file: walk count 0 (Backup.cpp:549-551)
+  const bool ok = write_work(t, f, dp_bits, range_start, range_end, keyx, keyy, total_count, total_time, 0) >= 0;
   return (fclose(f) == 0 && ok) ? 0 : -1;
+}
+
+int kgi_save_work_walks(kgi_table* t, const char* path, uint32_t dp_bits, const uint64_t range_start[4], const uint64_t range_end[4],
+                        const uint64_t keyx[4], const uint64_t keyy[4], uint64_t total_count, double total_time,
+                        uint64_t total_walks, uint64_t* walk_offset) {
+  FILE* f = fopen(path, "wb");
+  if (!f) return -1;
+  const long long off = write_work(t, f, dp_bits, range_start, range_end, keyx, keyy, total_count, total_time, total_walks);
+  bool ok = off >= 0 && fflush(f) == 0;
+  // the walk records are written later, possibly by other processes with pwrite: give the file its final length now
+  ok = ok && ftruncate(fileno(f), (off_t)(off + (long long)total_walks * KGI_WALK_SIZE)) == 0;
+  if (fclose(f) != 0 || !ok) return -1;
+  if (walk_offset) *walk_offset = (uint64_t)off;
+  return 0;
 }
 
 int kgi_load_work(kgi_table* t, const char* path, uint32_t* dp_bits, uint64_t* total_count, double* total_time) {
@@ -393,6 +418,56 @@ int kgi_load_work(kgi_table* t, const char* path, uint32_t* dp_bits, uint64_t* t
   if (dp_bits) *dp_bits = dp;
   if (total_count) *total_count = cnt;
   if (total_time) *total_time = tm;
+  return 0;
+}
+
+// Kangaroo::LoadWork (Backup.cpp:154-200) plus the walk count that follows the table.  t == NULL reads the header and
+// skips the table (what every rank but the table's owner needs on resume).
+int kgi_load_work_ex(kgi_table* t, const char* path, uint32_t* dp_bits, uint64_t range_start[4], uint64_t range_end[4],
+                     uint64_t keyx[4], uint64_t keyy[4], uint64_t* total_count, double* total_time,
+                     uint64_t* n_walks, uint64_t* walk_offset) {
+  FILE* f = fopen(path, "rb");
+  if (!f) return -1;
+  uint32_t head = 0, version = 0, dp = 0;
+  U256 rs, re, kx, ky;
+  uint64_t cnt = 0, nw = 0; double tm = 0;
+  bool ok = fread(&head, 4, 1, f) == 1 && fread(&version, 4, 1, f) == 1 && head == HEADW_MAGIC;
+  ok = ok && fread(&dp, 4, 1, f) == 1 && fread(rs.v, 32, 1, f) == 1 && fread(re.v, 32, 1, f) == 1;
+  ok = ok && fread(kx.v, 32, 1, f) == 1 && fread(ky.v, 32, 1, f) == 1 && fread(&cnt, 8, 1, f) == 1 && fread(&tm, 8, 1, f) == 1;
+  int rc = ok ? 0 : -1;
+  if (ok) {                                                       // Backup.cpp:175-179: the key must lie on the curve
+    const U256 seven = {{7, 0, 0, 0}};
+    const bool canon = !geq(kx, FP) && !geq(ky, FP);
+    if (!canon || !eq(fmul(ky, ky), add_mod(fmul(fmul(kx, kx), kx), seven, FP))) { ok = false; rc = -2; }
+  }
+  long long pos = 156;
+  if (t) table_reset(t);
+  for (uint32_t h = 0; ok && h < HASH_SIZE; h++) {
+    uint32_t nb = 0, cap = 0;
+    ok = fread(&nb, 4, 1, f) == 1 && fread(&cap, 4, 1, f) == 1;
+    if (!ok) break;
+    if (t) {
+      Bucket& b = t->buckets[h];
+      b.cap = cap;
+      b.items.resize(nb);
+      ok = fread(b.items.data(), sizeof(Entry), nb, f) == nb;
+    } else {
+      ok = fseeko(f, (off_t)sizeof(Entry) * nb, SEEK_CUR) == 0;
+    }
+    pos += 8 + (long long)sizeof(Entry) * nb;
+  }
+  ok = ok && fread(&nw, 8, 1, f) == 1;
+  fclose(f);
+  if (!ok) { if (t) table_reset(t); return rc ? rc : -1; }
+  if (dp_bits) *dp_bits = dp;
+  if (range_start) memcpy(range_start, rs.v, 32);
+  if (range_end) memcpy(range_end, re.v, 32);
+  if (keyx) memcpy(keyx, kx.v, 32);
+  if (keyy) memcpy(keyy, ky.v, 32);
+  if (total_count) *total_count = cnt;
+  if (total_time) *total_time = tm;
+  if (n_walks) *n_walks = nw;
+  if (walk_offset) *walk_offset = (uint64_t)(pos + 8);
   return 0;
 }
 

@@ -15,6 +15,7 @@ NB_JUMP = 32        # Constants.h:29
 GPU_GRP_SIZE = 128  # Constants.h:32
 NB_RUN = 64         # Constants.h:35
 TAME, WILD = 0, 1   # Constants.h:38-39
+WALK_SIZE = 96      # work-file kangaroo record {x[4], y[4], d[4]} (Backup.cpp:535-545)
 ORDER = 0xFFFFFFFFFFFFFFFFFFFFFFFFFFFFFFFEBAAEDCE6AF48A03BBFD25E8CD0364141
 _M64 = 0xFFFFFFFFFFFFFFFF
 _u64p = ctypes.POINTER(ctypes.c_uint64)
@@ -230,6 +231,55 @@ class GPUEngine:
         assert sc.shape[0] == n and ad.shape[0] == n
         kx, ky = _limbs([key[0]], 4), _limbs([key[1]], 4)
         self._ck(self._lib.kgx_create_herd(self._h, _p(sc), _p(ad), _p(kx), _p(ky), TAME), "CreateHerd")
+
+    # -- work-file walks (kgx_walks_*: 96-byte {x[4], y[4], d[4]} records, d unbiased mod n) ----------------------
+    def _wo(self):
+        return _limbs([self.wildOffset & ((1 << 128) - 1)], 2)
+
+    def WalksBegin(self):
+        """Convert the herd into work-file records on the device, after the launch in flight; returns at once."""
+        self._ck(self._lib.kgx_walks_begin(self._h, _p(self._wo())), "WalksBegin")
+
+    def WalksRead(self, out, first=0, count=None):
+        """Copy records [first, first + count) of the pending export into `out` (writable buffer of count * 96 bytes:
+        numpy uint8 array or pinned torch tensor).  Waits for the export only."""
+        count = self.nbKangaroo - first if count is None else count
+        a = out if isinstance(out, np.ndarray) else None
+        ptr = a.ctypes.data if a is not None else out.data_ptr()
+        nbytes = a.nbytes if a is not None else out.numel() * out.element_size()
+        assert nbytes >= count * WALK_SIZE
+        self._ck(self._lib.kgx_walks_read(self._h, ctypes.c_void_p(ptr), int(first), int(count)), "WalksRead")
+        return out
+
+    def WalksEnd(self):
+        self._ck(self._lib.kgx_walks_end(self._h), "WalksEnd")
+
+    def GetWalks(self):
+        """The whole herd as an (n, 12) uint64 array of work-file records (begin + read + end)."""
+        out = np.empty((self.nbKangaroo, 12), dtype=np.uint64)
+        self.WalksBegin()
+        try:
+            self.WalksRead(out.view(np.uint8).reshape(-1))
+        finally:
+            self.WalksEnd()
+        return out
+
+    def LoadWalks(self, recs, key=None, verify=True, bad_cap=None):
+        """Write `recs` ((count, 12) uint64 or count * 96 uint8 records, count <= nbKangaroo) to kIdx [0, count); the rest
+        of the herd is left as it is.  verify: check d*G (tame) / key + d*G (wild) for every record -> (n_bad, bad
+        indices (ascending, at most bad_cap)); (0, empty) without verification."""
+        a = np.ascontiguousarray(recs).view(np.uint8).reshape(-1)
+        assert a.size % WALK_SIZE == 0
+        count = a.size // WALK_SIZE
+        if verify and key is None:
+            raise ValueError("LoadWalks: verification needs the key")
+        kx, ky = (_limbs([key[0]], 4), _limbs([key[1]], 4)) if key is not None else (np.zeros((1, 4), np.uint64), np.zeros((1, 4), np.uint64))
+        cap = count if bad_cap is None else int(bad_cap)
+        bad = np.zeros(max(cap, 1), dtype=np.uint64)
+        nb = ctypes.c_uint64(0)
+        self._ck(self._lib.kgx_walks_load(self._h, ctypes.c_void_p(a.ctypes.data), count, _p(self._wo()), _p(kx), _p(ky),
+                                          int(bool(verify)), ctypes.byref(nb), _p(bad), ctypes.c_uint32(min(cap, 0xFFFFFFFF))), "LoadWalks")
+        return int(nb.value), bad[:min(nb.value, cap)].copy()
 
     def callKernel(self):
         """GPUEngine.cu:540-557."""

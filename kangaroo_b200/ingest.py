@@ -13,6 +13,7 @@ from ._lib import INGEST_PATH as LIB_PATH
 
 EV_RESET, EV_COLLISION = 1, 2
 DP40_BYTES, ITEM_BYTES = 40, 56
+WALK_BYTES = 96          # work-file kangaroo record {x[4], y[4], d[4]}
 _M64 = 0xFFFFFFFFFFFFFFFF
 
 
@@ -38,6 +39,10 @@ _SIGS = {
                                      ctypes.c_double]),
     "kgi_load_work": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.POINTER(ctypes.c_uint32), _u64p,
                                      ctypes.POINTER(ctypes.c_double)]),
+    "kgi_save_work_walks": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_uint32, _u64p, _u64p, _u64p, _u64p,
+                                           ctypes.c_uint64, ctypes.c_double, ctypes.c_uint64, _u64p]),
+    "kgi_load_work_ex": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.POINTER(ctypes.c_uint32), _u64p, _u64p, _u64p, _u64p,
+                                        _u64p, ctypes.POINTER(ctypes.c_double), _u64p, _u64p]),
 }
 EXPORTED_SYMBOLS = sorted(_SIGS)
 _lib = None
@@ -60,6 +65,39 @@ def load_library():
 
 def _limbs4(v):
     return (ctypes.c_uint64 * 4)(*[(int(v) >> (64 * k)) & _M64 for k in range(4)])
+
+
+def _int4(a):
+    return sum(int(a[k]) << (64 * k) for k in range(4))
+
+
+class WorkInfo:
+    """Header of a HEADW work file (Backup.cpp:154-200) plus where its kangaroos are."""
+    __slots__ = ("path", "dp_bits", "range_start", "range_end", "key", "total_count", "total_time", "n_walks", "walk_offset")
+
+    def __init__(self, **kw):
+        for k, v in kw.items():
+            setattr(self, k, v)
+
+    def __repr__(self):
+        return "WorkInfo(%s)" % ", ".join("%s=%r" % (k, getattr(self, k)) for k in self.__slots__)
+
+
+def read_work_info(path, table=None):
+    """Read a work file's header and walk count (kgi_load_work_ex); load its DP table into `table` (a DPTable) when
+    given, else skip the table.  Raises ValueError when the key is not on the curve."""
+    lib = load_library()
+    dp, cnt, tm = ctypes.c_uint32(0), ctypes.c_uint64(0), ctypes.c_double(0)
+    rs, re, kx, ky = ((ctypes.c_uint64 * 4)() for _ in range(4))
+    nw, off = ctypes.c_uint64(0), ctypes.c_uint64(0)
+    rc = lib.kgi_load_work_ex(table._h if table is not None else None, os.fsencode(path), ctypes.byref(dp), rs, re, kx, ky,
+                              ctypes.byref(cnt), ctypes.byref(tm), ctypes.byref(nw), ctypes.byref(off))
+    if rc == -2:
+        raise ValueError("%s: key does not lie on the elliptic curve" % path)
+    if rc != 0:
+        raise RuntimeError("kgi_load_work_ex: %s is not a HEADW work file" % path)
+    return WorkInfo(path=path, dp_bits=dp.value, range_start=_int4(rs), range_end=_int4(re), key=(_int4(kx), _int4(ky)),
+                    total_count=cnt.value, total_time=tm.value, n_walks=nw.value, walk_offset=off.value)
 
 
 class DPTable:
@@ -135,6 +173,21 @@ class DPTable:
                                      _limbs4(pubkey[0]), _limbs4(pubkey[1]), int(total_count), float(total_time))
         if rc != 0:
             raise RuntimeError("kgi_save_work: cannot write %s" % path)
+
+    def save_work_walks(self, path, dp_bits, range_start, range_end, pubkey, total_count, total_time, total_walks):
+        """save_work with `total_walks` kangaroo records to follow; the file already has its final size.  Returns the byte
+        offset of the first walk record."""
+        off = ctypes.c_uint64(0)
+        rc = self._lib.kgi_save_work_walks(self._h, os.fsencode(path), int(dp_bits), _limbs4(range_start), _limbs4(range_end),
+                                           _limbs4(pubkey[0]), _limbs4(pubkey[1]), int(total_count), float(total_time),
+                                           int(total_walks), ctypes.byref(off))
+        if rc != 0:
+            raise RuntimeError("kgi_save_work_walks: cannot write %s" % path)
+        return off.value
+
+    def load_work_ex(self, path):
+        """load_work returning the whole header (WorkInfo)."""
+        return read_work_info(path, self)
 
     def load_work(self, path):
         dp, cnt, tm = ctypes.c_uint32(0), ctypes.c_uint64(0), ctypes.c_double(0)

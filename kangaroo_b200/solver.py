@@ -1,8 +1,10 @@
 """Stand-alone multi-GPU driver of the jump engine: the role Kangaroo::Run / SolveKeyGPU (Kangaroo.cpp:913-1083,
 510-644) plays in the reference, with the reference's TCP client/server (Network.cpp) replaced in-box by one process
-per GPU and an NCCL gather of the DP records to rank 0 (kangaroo_b200/dist.py).  Kept deliberately small: it exists to
-exercise the engine end to end (BASELINE config 4) -- the full-featured caller remains the reference's own program
-linked against the engine (INTEGRATION.md).
+per GPU and an NCCL gather of the DP records to rank 0 (kangaroo_b200/dist.py).  Small on purpose -- it exists to run the
+engine end to end at full multi-GPU speed (BASELINE config 4), and the full-featured caller remains the reference's own
+program linked against the engine (INTEGRATION.md) -- except for checkpoints: a run of days must survive preemption, so it
+writes and resumes the reference's work files, kangaroos included (-w / -wi / -ws / -i there, --work-file /
+--work-interval / --save-kangaroos / --resume here).
 
 Per step (= one GPUEngine::Launch on every rank) nothing on the data path is Python:
   engine      kgx_collect(cap=0, relaunch=1): wait for launch i, start launch i+1, no host copy of records
@@ -13,15 +15,30 @@ Per step (= one GPUEngine::Launch on every rank) nothing on the data path is Pyt
               -> events: KGI_EV_COLLISION -> kgi_resolve (CollisionCheck/CheckKey with the reference's Secp256K1)
                          KGI_EV_RESET     -> (rank, kIdx) sent back to the owner, which re-creates that kangaroo
                                              (Kangaroo.cpp:601-609: CreateHerd(1) + SetKangaroo)
-  all ranks   one small broadcast: [stop, n_resets, (rank, kIdx) ...]
+  all ranks   one small broadcast: [stop, n_resets, checkpoint begin, checkpoint offset, (rank, kIdx) ...]
+
+Checkpoints (kangaroo_b200/checkpoint.py for the file protocol).  The table in a checkpoint holds exactly the DPs of
+launches 1..L, its walks are the herd after launch L on every rank and its count the jumps through launch L:
+  step s      rank 0 decides, the control word carries "begin"; every rank calls kgx_walks_begin, which converts the
+              herd on the device in stream order behind launch L = s + 1 (in flight) and returns at once
+  step s + 1  launch L's records go to the ingest thread and rank 0 queues a save marker right behind them: the ingest
+              thread writes header + table to F.tmp (the step loop stalls only if this outlasts the next step's insert)
+  later       the walk offset goes out in a control word; every rank's writer thread copies its walks out in chunks and
+              pwrites them; a MIN all-reduce of the ranks' done flags runs each step until all are written; rank 0 then
+              fsyncs and renames F.tmp -> F
+When the run stops without a key (--max-steps, SIGINT, SIGTERM) the launch in flight is collected too and a last
+checkpoint is written the same way, synchronously.
 
   single GPU :  python -m kangaroo_b200.solver in.txt --dp 12
   N GPUs     :  torchrun --nproc-per-node N -m kangaroo_b200.solver in.txt --dp 12
+  checkpoint :  ... --work-file run.work --work-interval 600 --save-kangaroos
+  resume     :  python -m kangaroo_b200.solver --resume run.work [--work-file run.work ...]
 """
 import argparse
 import ctypes
 import os
 import queue
+import signal
 import sys
 import threading
 import time
@@ -29,12 +46,34 @@ import time
 import numpy as np
 
 from . import ecmath as ec
-from .engine import GPUEngine, NB_JUMP, NB_RUN, WILD, random_herd_arrays
+from . import checkpoint as ckpt
+from .engine import GPUEngine, NB_JUMP, NB_RUN, WILD, WALK_SIZE, random_herd_arrays
 from .dist import DPGather, SlabView, DP40_BYTES
-from .ingest import DPTable, EV_RESET, EV_COLLISION
+from .ingest import DPTable, EV_RESET, EV_COLLISION, read_work_info
 
 ORDER = ec.N
 MAX_RESETS = 255          # per step, carried in the control broadcast
+CTRL_HEAD = 4             # control word: stop, n_resets, checkpoint begin, checkpoint walk offset (-1: table write failed)
+STOP_KEY, STOP_SIGNAL = 1, 2
+WALK_CHUNK = 1 << 18      # walks per pinned chunk of a checkpoint writer (24 MiB)
+
+_signalled = []           # SIGINT / SIGTERM received (main() installs the handler)
+
+
+def _on_signal(signum, frame):
+    _signalled.append(signum)
+
+
+class _Checkpoint:
+    """One checkpoint in progress on this rank."""
+
+    def __init__(self, path, final):
+        self.path, self.final = path, final
+        self.phase = "exported"          # -> "table" (marker queued, rank 0) -> "writing" (offset known)
+        self.t0 = time.time()
+        self.result = queue.Queue()      # rank 0: walk offset from the ingest thread (or an exception)
+        self.writer = None
+        self.stall0 = 0.0
 
 
 def create_jump_table(range_power):
@@ -65,7 +104,8 @@ def dp_mask(bits):
 
 
 class Solver:
-    def __init__(self, start, end, pub, dp_bits, grid=None, max_found=1 << 17, seed=None, ingest_threads=0):
+    def __init__(self, start, end, pub, dp_bits, grid=None, max_found=1 << 17, seed=None, ingest_threads=0,
+                 work_file="", work_interval=0.0, save_kangaroos=False, resume=None):
         import torch
         self.torch = torch
         self.rank = int(os.environ.get("RANK", "0"))
@@ -96,13 +136,16 @@ class Solver:
         self.eng.CreateHerdRaw(sc, d128, self.key)
         self.gather = DPGather(self.eng, self.dist, self.rank, self.world, torch, wire="dp40") if self.world > 1 else None
         self.dps = DPTable(threads=ingest_threads) if self.rank == 0 else None      # rank 0: the reference HashTable
+        self.work_file, self.work_interval, self.save_kangaroos = work_file, float(work_interval or 0), bool(save_kangaroos)
+        self.jumps0, self.time0 = 0, 0.0
+        self.loaded = self.bad = 0
         # Two pinned staging buffers: while the ingest thread inserts step k's records, step k+1's land in the other one.  The
         # NCCL kernels of a step cannot start before the jump launch that occupies every SM has finished, so without this
         # decoupling the CPU insert (3-4 ms at 8 GPUs) sat exposed between two launches: 97 instead of 112 GJump/s.
         self._hosts = ([torch.empty(self.world * max_found * DP40_BYTES, dtype=torch.uint8).pin_memory() for _ in range(2)]
                        if self.rank == 0 else None)
         self._hidx = 0
-        self._work = queue.Queue(maxsize=1)
+        self._work = queue.Queue()          # steps' records (at most two in flight, _staging) and checkpoint markers
         self._done = queue.Queue()
         self._pending = 0
         self._acc_found, self._acc_resets = None, []
@@ -110,12 +153,23 @@ class Solver:
         if self.rank == 0:
             self._thread = threading.Thread(target=self._ingest_loop, daemon=True)
             self._thread.start()
-        self._ctrl = torch.zeros(2 + 2 * MAX_RESETS, dtype=torch.int64, device="cuda")
-        self.jumps = 0
+        self._ctrl = torch.zeros(CTRL_HEAD + 2 * MAX_RESETS, dtype=torch.int64, device="cuda")
+        self._flag = torch.zeros(1, dtype=torch.int64, device="cuda")
+        self.jumps = self.jumps0
+        self.stop_reason = 0
+        self._ck = None
+        self._ck_last = time.time()
+        self._ck_host = None
+        self.t_stall = 0.0                  # step loop blocked by checkpoints: export set-up + waits behind the table write
+        self._table_busy = False            # ingest thread is writing a checkpoint's header and table
+        self.checkpoints = []               # rank 0: (path, bytes, seconds, stall seconds) of every committed checkpoint
         self.same_herd = 0
         self.resets_done = 0
         self.t_ingest = 0.0
         self.stop = False
+        if resume:
+            self._resume(resume, n)
+            self.jumps = self.jumps0
 
     # -- rank 0: ingest -------------------------------------------------------------------------------------------
     def _ingest(self, segments):
@@ -140,7 +194,23 @@ class Solver:
             segs = self._work.get()
             if segs is None:
                 return
+            if isinstance(segs, _Checkpoint):
+                self._write_table(segs)
+                continue
             self._done.put(self._ingest(segs))
+
+    def _write_table(self, ck):
+        """ingest thread, at the save marker: every DP of launches 1..L is in the table, none of a later launch"""
+        self._table_busy = True
+        try:
+            walks = self.eng.nbKangaroo * self.world if self.save_kangaroos else 0
+            off = self.dps.save_work_walks(ckpt.tmp_path(ck.path), self.dp_bits, self.start, self.end, self.pub,
+                                           total_count=ck.count, total_time=ck.time, total_walks=walks)
+            ck.result.put(off)
+        except BaseException as e:
+            ck.result.put(e)
+        finally:
+            self._table_busy = False
 
     def _submit(self, segs):
         """hand one step's records to the ingest thread"""
@@ -149,8 +219,11 @@ class Solver:
 
     def _staging(self):
         """the staging buffer for this step; at most one older step may still be in the ingest thread (it reads the OTHER buffer)"""
+        t0 = time.perf_counter() if self._table_busy else None   # only a wait that starts behind a table write is its cost
         while self._pending >= 2:
             self._take(block=True)
+        if t0 is not None:
+            self.t_stall += time.perf_counter() - t0
         host = self._hosts[self._hidx]
         self._hidx ^= 1
         return host
@@ -185,10 +258,11 @@ class Solver:
         self.eng.SetKangaroo(kidx, pos[0], pos[1], d)
         self.resets_done += 1
 
-    def step(self):
-        """one Launch on every rank; returns the private key on rank 0 when found (None otherwise)"""
+    def step(self, relaunch=True):
+        """one Launch on every rank; returns the private key on rank 0 when found (None otherwise).  relaunch=False
+        collects the launch in flight without starting another (the last step before a final checkpoint)."""
         torch = self.torch
-        n_found = self.eng.collect_count(relaunch=True)                  # launch i done, launch i+1 running
+        n_found = self.eng.collect_count(relaunch=relaunch)              # launch i done, launch i+1 running
         cnt = min(n_found, self.eng.maxFound)
         self.jumps += self.eng.nbKangaroo * NB_RUN * self.world
         found, resets = None, []
@@ -210,29 +284,230 @@ class Solver:
                 host[:cnt * DP40_BYTES].copy_(dev, non_blocking=True)
                 torch.cuda.current_stream().synchronize()
                 self._submit([(0, host.numpy()[:cnt * DP40_BYTES])])
+        ck_begin, ck_off = 0, 0
         if self.rank == 0:
+            self._ck_marker()                                               # right behind launch L's records
             found, resets = self._harvest()
-        # control word: stop flag + kangaroos to re-create, back to their owners
+            stop = STOP_KEY if found is not None else (STOP_SIGNAL if _signalled else 0)
+            if (self._ck is None and self.work_file and self.work_interval > 0 and not stop and relaunch
+                    and time.time() - self._ck_last >= self.work_interval):
+                ck_begin = 1
+            ck_off = self._ck_offset(block=False)
+        # control word: stop flag, checkpoint, kangaroos to re-create, back to their owners
         if self.dist is not None:
             if self.rank == 0:
                 resets = resets[:MAX_RESETS]
-                c = [1 if found is not None else 0, len(resets)] + [v for rk in resets for v in rk]
+                c = [stop, len(resets), ck_begin, ck_off] + [v for rk in resets for v in rk]
                 self._ctrl[:len(c)].copy_(torch.tensor(c, dtype=torch.int64))
             self.dist.broadcast(self._ctrl, 0)
-            c = self._ctrl.cpu().tolist()
-            self.stop = bool(c[0])
-            resets = [(c[2 + 2 * i], c[3 + 2 * i]) for i in range(c[1])]
-        else:
-            self.stop = found is not None
+            c = self._ctrl[:CTRL_HEAD + 2 * MAX_RESETS].cpu().tolist()
+            stop, ck_begin, ck_off = c[0], c[2], c[3]
+            resets = [(c[CTRL_HEAD + 2 * i], c[CTRL_HEAD + 1 + 2 * i]) for i in range(c[1])]
+        self.stop_reason = stop
+        self.stop = bool(stop)
+        if ck_begin:
+            self._ck_begin(final=False)
+        if ck_off:
+            self._ck_write(ck_off)
+        if self._ck is not None and self._ck.phase == "writing":
+            self._ck_poll_done(block=False)
+        # A kangaroo reset below was exported by a checkpoint begun in this step as it was before the reset: on resume it
+        # re-emits a DP the table already holds and is reset again -- harmless.
         for rk, kidx in resets:
             self.same_herd += 1
             if rk == self.rank and not self.stop:
                 self._reset_kangaroo(kidx)
         return found
 
+    # -- checkpoints ------------------------------------------------------------------------------------------------
+    def _ck_begin(self, final):
+        """every rank, in the same step: export the herd behind the launch in flight (or, final, the last launch)"""
+        t0 = time.perf_counter()
+        self._ck = _Checkpoint(self.work_file, final)
+        self._ck.stall0 = self.t_stall
+        if self.save_kangaroos:
+            self.eng.WalksBegin()
+        self.t_stall += time.perf_counter() - t0
+
+    def _ck_marker(self):
+        """rank 0, after submitting the records of launch L: queue the table write behind them"""
+        ck = self._ck
+        if ck is None or ck.phase != "exported":
+            return
+        ck.count = self.jumps
+        ck.time = self.time0 + (time.time() - self._t_run)
+        ck.phase = "table"
+        self._work.put(ck)
+
+    def _ck_offset(self, block):
+        """rank 0: the walk offset once the ingest thread wrote header and table (0 while pending, -1 on failure)"""
+        ck = self._ck
+        if ck is None or ck.phase != "table" or getattr(ck, "offset", None) is not None:
+            return 0
+        try:
+            r = ck.result.get(block=block)
+        except queue.Empty:
+            return 0
+        if isinstance(r, BaseException):
+            print("checkpoint: cannot write %s: %s" % (ckpt.tmp_path(ck.path), r), flush=True)
+            r = -1
+        ck.offset = r
+        return r
+
+    def _ck_write(self, offset):
+        """every rank: start writing this rank's walks at the offset rank 0 announced"""
+        ck = self._ck
+        ck.phase = "writing"
+        if offset < 0:
+            ck.failed = True
+            return
+        if not self.save_kangaroos:
+            return
+        n = self.eng.nbKangaroo
+        if self._ck_host is None:
+            self._ck_host = self.torch.empty(min(WALK_CHUNK, n) * WALK_SIZE, dtype=self.torch.uint8).pin_memory()
+        host = self._ck_host
+        eng = self.eng
+
+        def read(buf, first, count):
+            eng.WalksRead(host, first, count)
+        ck.writer = ckpt.SliceWriter(ckpt.tmp_path(ck.path), offset, self.rank * n, n, read, host.numpy(), min(WALK_CHUNK, n),
+                                     on_exit=eng.WalksEnd)
+
+    def _ck_local_state(self):
+        ck = self._ck
+        if getattr(ck, "failed", False):
+            return -1
+        return ck.writer.state if ck.writer is not None else 1
+
+    def _ck_poll_done(self, block):
+        """every rank, in the same step: have all ranks written their walks?  rank 0 then commits the file"""
+        ck = self._ck
+        if block and ck.writer is not None:
+            ck.writer.join()
+        st = self._ck_local_state()
+        if self.dist is not None:
+            self._flag.fill_(st)
+            self.dist.all_reduce(self._flag, op=self.dist.ReduceOp.MIN)
+            st = int(self._flag.item())
+        if st == 0:
+            return
+        self._ck_release(ck)
+        if self.rank == 0:
+            if st == 1:
+                ckpt.commit(ck.path)
+                size = os.path.getsize(ck.path)
+                dt, stall = time.time() - ck.t0, self.t_stall - ck.stall0
+                self.checkpoints.append((ck.path, size, dt, stall))
+                print("checkpoint: %s  %.1f MB  %.2f s  (step loop waited %.3f s)" % (ck.path, size / 1e6, dt, stall), flush=True)
+            else:
+                ckpt.discard(ck.path)
+                print("checkpoint: %s not written, the previous file is kept" % ck.path, flush=True)
+        self._ck = None
+        self._ck_last = time.time()
+
+    def _ck_release(self, ck):
+        """this rank's side of a checkpoint that is over: writer joined, export ended (also when no writer ran, e.g. after a
+        failed table write), so the next checkpoint can begin"""
+        if ck.writer is not None:
+            ck.writer.join()
+            if ck.writer.error is not None:
+                print("checkpoint: rank %d could not write its walks: %s" % (self.rank, ck.writer.error), flush=True)
+        elif self.save_kangaroos:
+            self.eng.WalksEnd()
+
+    def _ck_abandon(self):
+        """the run ends with a checkpoint in progress (the key was found): finish what is running on this rank -- the walk
+        writer, the table write queued on rank 0 -- before the engine and the table go away, and drop F.tmp.  Local only:
+        no collective, every rank does the same."""
+        ck = self._ck
+        if ck is None:
+            return
+        self._ck_release(ck)
+        if self.rank == 0:
+            if ck.phase == "table" and getattr(ck, "offset", None) is None:
+                ck.result.get()                             # the ingest thread is writing or about to write the table
+            ckpt.discard(ck.path)
+            print("checkpoint: %s abandoned, the run ended while it was written; the previous file is kept" % ck.path, flush=True)
+        self._ck = None
+
+    def _ck_finish(self):
+        """every rank: drive the checkpoint in progress to its end, blocking"""
+        ck = self._ck
+        if ck is None:
+            return
+        if self.rank == 0:
+            self._ck_marker()
+        if ck.phase != "writing":
+            off = self._ck_offset(block=True) if self.rank == 0 else 0
+            if self.dist is not None:
+                self._flag.fill_(off)
+                self.dist.broadcast(self._flag, 0)
+                off = int(self._flag.item())
+            self._ck_write(off)
+        self._ck_poll_done(block=True)
+
+    def final_checkpoint(self):
+        """the run stopped without a key: collect the launch in flight, then write a checkpoint of the state after it"""
+        key = self.step(relaunch=False)
+        if self.stop_reason == STOP_KEY:
+            return key
+        self._ck_finish()                                   # a periodic checkpoint still in progress
+        self._ck_begin(final=True)
+        self._ck_finish()
+        return None
+
+    # -- resume -----------------------------------------------------------------------------------------------------
+    def _resume(self, path, n):
+        """Kangaroo::LoadWork + FectchKangaroos (Backup.cpp:154-200, 291-359): rank 0 takes the table, every rank its slice
+        of the walks; the herd created above keeps the kangaroos the file lacks."""
+        info = read_work_info(path, self.dps)          # rank 0 loads the table, the other ranks skip it
+        self.jumps0, self.time0 = info.total_count, info.total_time
+        first = self.rank * n
+        count = max(0, min(n, info.n_walks - first))
+        err = None
+        try:
+            if count:
+                err = self._load_slice(info, first, count, n)
+            elif self.rank == 0:
+                print("resume: no walks in %s, %d kangaroos created fresh per GPU" % (info.path, n), flush=True)
+        except Exception as e:                              # e.g. an unreadable file, a failed device call
+            err = "resume: rank %d: %s" % (self.rank, e)
+        if self.dist is not None:                           # every rank stops when one cannot go on, none waits in a collective
+            self._flag.fill_(0 if err else 1)
+            self.dist.all_reduce(self._flag, op=self.dist.ReduceOp.MIN)
+            if not err and int(self._flag.item()) == 0:
+                err = "resume: rank %d: another rank could not resume from %s" % (self.rank, info.path)
+        if err:
+            raise SystemExit(err)
+        left = info.n_walks - self.world * n
+        if self.rank == 0 and left > 0:
+            print("FectchKangaroos: Warning %d unhandled kangaroos !" % left, flush=True)
+
+    def _load_slice(self, info, first, count, n):
+        """this rank's walks [first, first + count) of the file into kIdx [0, count), checked; -> error text or None"""
+        recs = np.fromfile(info.path, dtype=np.uint8, count=count * WALK_SIZE, offset=info.walk_offset + first * WALK_SIZE)
+        if recs.size != count * WALK_SIZE:
+            return "resume: %s is truncated (walks of rank %d missing)" % (info.path, self.rank)
+        t0 = time.time()
+        nbad, bad = self.eng.LoadWalks(recs, key=self.key, verify=True)
+        # tame walks (d*G) are valid for any key: a file of another key fails on the wild half only
+        bad_wild = int(np.count_nonzero(bad & 1))
+        if 2 * nbad > count or 2 * bad_wild > count // 2:
+            return ("resume: %d of %d walks (%d wild) of %s fail d*G (+key) = position: the file does not belong to this key "
+                    "and range" % (nbad, count, bad_wild, info.path))
+        for kidx in bad:
+            self._reset_kangaroo(int(kidx))
+        self.loaded, self.bad = count, nbad
+        print("resume: rank %d: %d walks loaded and checked in %.2f s, %d re-created, %d created fresh" %
+              (self.rank, count, time.time() - t0, nbad, n - count), flush=True)
+        return None
+
     def run(self, max_steps=1 << 30, verbose=True):
         self.eng.callKernel()
         t0 = time.time()
+        self._t_run = t0
+        self._ck_last = t0
         key = None
         steps = 0
         self.steady = None                      # (time, jumps) after the first 32 steps: NCCL communicator set-up, first table growth
@@ -244,20 +519,28 @@ class Solver:
             if verbose and self.rank == 0 and (s % 64 == 63 or self.stop):
                 dt = time.time() - t0
                 print("[%6.1fs] 2^%.2f jumps  %.0f MJump/s  %d DPs  dead %d  ingest %.1f ms/step" %
-                      (dt, np.log2(max(self.jumps, 1)), self.jumps / dt / 1e6, len(self.dps), self.same_herd,
-                       1e3 * self.t_ingest / steps), flush=True)
+                      (self.time0 + dt, np.log2(max(self.jumps, 1)), (self.jumps - self.jumps0) / dt / 1e6, len(self.dps),
+                       self.same_herd, 1e3 * self.t_ingest / steps), flush=True)
             if self.stop:
                 break
+        t_loop, jumps_loop = time.time(), self.jumps           # the steady rate leaves the last checkpoint out
+        if self.work_file and self.stop_reason != STOP_KEY:
+            k = self.final_checkpoint()
+            steps += 1
+            key = key if key is not None else k
+        self._ck_abandon()
         self.eng.sync()
         if self.rank == 0 and key is None:                      # the last steps' records may still be in the ingest thread
             key, _ = self._harvest(wait_all=True)
         t1 = time.time()
         self.elapsed = t1 - t0
         self.steps = steps
-        self.steady_rate = ((self.jumps - self.steady[1]) / (t1 - self.steady[0]) if self.steady and steps > 64 else self.jumps / self.elapsed)
+        self.steady_rate = ((jumps_loop - self.steady[1]) / (t_loop - self.steady[0]) if self.steady and steps > 64
+                            else (self.jumps - self.jumps0) / self.elapsed)
         return key
 
     def close(self):
+        self._ck_abandon()
         if self._thread is not None:
             self._harvest(wait_all=True)
             self._work.put(None)
@@ -270,35 +553,61 @@ class Solver:
 
 def main(argv=None):
     ap = argparse.ArgumentParser()
-    ap.add_argument("config")
-    ap.add_argument("--dp", type=int, default=12)
+    ap.add_argument("config", nargs="?", default=None, help="range start, range end, public keys (not needed with --resume)")
+    ap.add_argument("--dp", type=int, default=None, help="distinguished-point bits (default 12, or the resumed file's)")
     ap.add_argument("--grid", default="")
     ap.add_argument("--seed", type=int, default=None)
     ap.add_argument("--max-steps", type=int, default=1 << 30)
     ap.add_argument("--ingest-threads", type=int, default=0, help="workers of the rank-0 DP table (0 = min(8, cores))")
     ap.add_argument("--save-work", default="", help="write the rank-0 DP table as a reference work file (HEADW) at the end")
+    ap.add_argument("--work-file", default="", help="write checkpoints (reference work files) to this file (reference -w)")
+    ap.add_argument("--work-interval", type=float, default=0.0,
+                    help="seconds between checkpoints (reference -wi); without it a checkpoint is written only when the run "
+                         "stops without the key (--max-steps, SIGINT, SIGTERM)")
+    ap.add_argument("--save-kangaroos", action="store_true", help="checkpoints include every rank's kangaroos (reference -ws)")
+    ap.add_argument("--resume", default="", help="continue from this work file: range, key, dp, count and time (reference -i)")
     a = ap.parse_args(argv)
-    start, end, pubs = ec.parse_config(a.config)
+    if a.resume:
+        info = read_work_info(a.resume)
+        start, end, pubs = info.range_start, info.range_end, [info.key]
+        dp = a.dp if a.dp is not None else info.dp_bits
+    elif a.config:
+        start, end, pubs = ec.parse_config(a.config)
+        dp = a.dp if a.dp is not None else 12
+    else:
+        ap.error("a config file or --resume is required")
+    if (a.work_interval or a.save_kangaroos) and not a.work_file:
+        ap.error("--work-interval and --save-kangaroos need --work-file")
     grid = tuple(int(v) for v in a.grid.split(",")) if a.grid else None
+    if a.work_file:
+        for sig in (signal.SIGINT, signal.SIGTERM):       # stop at the next step and write a last checkpoint
+            signal.signal(sig, _on_signal)
     rc = 0
     for i, pub in enumerate(pubs):
-        s = Solver(start, end, pub, a.dp, grid, seed=a.seed, ingest_threads=a.ingest_threads)
+        s = Solver(start, end, pub, dp, grid, seed=a.seed, ingest_threads=a.ingest_threads, work_file=a.work_file,
+                   work_interval=a.work_interval, save_kangaroos=a.save_kangaroos, resume=a.resume or None)
         if s.rank == 0:
             print("Range width: 2^%d  kangaroos/GPU: %d  GPUs: %d  dp: %d  ingest threads: %d" %
-                  (s.range_power, s.eng.nbKangaroo, s.world, a.dp, s.dps.threads), flush=True)
+                  (s.range_power, s.eng.nbKangaroo, s.world, dp, s.dps.threads), flush=True)
+            if a.resume:
+                print("resume: %s  count 2^%.2f  time %.1f s" % (a.resume, np.log2(max(s.jumps0, 1)), s.time0), flush=True)
         key = s.run(a.max_steps)
         if s.rank == 0:
             print("Solver rate: %.0f MJump/s steady state (after the first 32 steps), %.0f MJump/s over all %d steps (%.2f s); "
                   "rank-0 ingest %.2f ms/step; %d DPs; %d dead kangaroos re-created" %
-                  (s.steady_rate / 1e6, s.jumps / s.elapsed / 1e6, s.steps, s.elapsed, 1e3 * s.t_ingest / max(s.steps, 1), len(s.dps), s.same_herd))
+                  (s.steady_rate / 1e6, (s.jumps - s.jumps0) / s.elapsed / 1e6, s.steps, s.elapsed, 1e3 * s.t_ingest / max(s.steps, 1),
+                   len(s.dps), s.same_herd))
+            print("Total count: %d jumps (2^%.2f)" % (s.jumps, np.log2(max(s.jumps, 1))))
             if a.save_work:
-                s.dps.save_work(a.save_work, a.dp, start, end, pub, total_count=s.jumps, total_time=s.elapsed)
+                s.dps.save_work(a.save_work, dp, start, end, pub, total_count=s.jumps, total_time=s.time0 + s.elapsed)
                 print("work file written: %s" % a.save_work)
             if key is not None and ec.mul(key) == pub:
                 print("Key#%2d Pub:  0x%064X\n       Priv: 0x%X" % (i, pub[0], key))
             else:
                 print("Key#%2d not found" % i); rc = 1
         s.close()
+        if _signalled:
+            break
     try:
         import torch.distributed as dist
         if dist.is_initialized():
