@@ -147,6 +147,50 @@ uint64_t kgx_kernel_launches(kgx_engine* e);
  * out = {serial section, modular inverse alone, parallel phase, tile-steps}; resets them. -1 when disabled. */
 int      kgx_debug_prof(kgx_engine* e, uint64_t out[4]);
 
+/* --- rank-0 distinguished-point table in device memory (SURVEY 8f row f1; kgx_dptable.cuh).  The decisions of the host
+ *     table's kgi_add (include/kgx_ingest.h: HashTable::Add) on records that are already on the device, and exports in
+ *     work-file order for kgi_fill_sorted.  Open addressing, linear probing, h-major home slots, 40 bytes per slot and at
+ *     most KGX_DPT_LOAD entries per slot: about 57 bytes per entry of capacity.
+ *   kgx_dpt_create        a table for `capacity` entries (at most kgx_dpt_max_capacity()) on device `dev`, collecting at
+ *                         most max_events events per insert; NULL on failure, text in kgx_dpt_last_error(NULL)
+ *   kgx_dpt_memory_bytes  device bytes such a table holds (export / load scratch included, insert scratch not: it grows
+ *                         to 12 bytes per record of the largest batch)
+ *   kgx_dpt_insert        stream-ordered on `stream` (a cudaStream_t; NULL = the legacy default stream): the 40-byte DP
+ *                         records of `nranks` ranks, rank r's counts[r] records at recs + r * stride * 40 (one rank:
+ *                         stride ignored, e.g. the records of kgx_convert_dps).  Records are decided in (rank, index)
+ *                         order like consecutive kgi_add calls.  At most two inserts may await kgx_dpt_events.
+ *   kgx_dpt_events        waits for the oldest pending insert and copies its events (KGX_DPT_EVENT_SIZE-byte kgi_event
+ *                         records, any order) to ev[0..cap); *n_ev = events produced (the excess over cap is dropped, as
+ *                         kgi_add), *entries = table entries after that insert.  0, -1 when a record had h >= 2^18
+ *                         (skipped, like kgi_add), -2 when a probe ran off the table, -3 on a CUDA or usage error.
+ *   kgx_dpt_count         entries after every insert queued so far (waits for them)
+ *   kgx_dpt_export_begin  snapshot point: the export holds the inserts queued before this call (stream-ordered behind them on
+ *                         `stream`); later inserts proceed and are not part of it
+ *   kgx_dpt_export_read   from any host thread: entries of buckets [first_bucket, first_bucket + k), k <= max_buckets as
+ *                         many as fit in entries_cap, sorted by (x[1], x[0]) inside each bucket, as 32-byte {x[2], d[2]}
+ *                         entries; counts[0..k) = entries per bucket.  k = 0 once first_bucket reaches 2^18.
+ *   kgx_dpt_export_end    ends the export
+ *   kgx_dpt_load          bulk load of distinct entries in work-file order (h[n], entries32 = n x 32 bytes; resume);
+ *                         synchronous, refused while inserts or an export are pending --- */
+typedef struct kgx_dpt kgx_dpt;
+#define KGX_DPT_EVENT_SIZE 48
+#define KGX_DPT_LOAD       0.7
+kgx_dpt*    kgx_dpt_create(int dev, uint64_t capacity, uint32_t max_events);
+void        kgx_dpt_destroy(kgx_dpt* t);
+const char* kgx_dpt_last_error(kgx_dpt* t);
+uint64_t    kgx_dpt_memory_bytes(uint64_t capacity);
+uint64_t    kgx_dpt_max_capacity(void);
+uint64_t    kgx_dpt_capacity(kgx_dpt* t);
+int         kgx_dpt_insert(kgx_dpt* t, const void* recs, uint32_t stride, const uint32_t* counts, uint32_t nranks, void* stream);
+int         kgx_dpt_events(kgx_dpt* t, void* ev, uint32_t cap, uint32_t* n_ev, uint64_t* entries);
+int         kgx_dpt_pending(kgx_dpt* t);
+int         kgx_dpt_count(kgx_dpt* t, uint64_t* entries);
+int         kgx_dpt_export_begin(kgx_dpt* t, void* stream);
+int         kgx_dpt_export_read(kgx_dpt* t, uint32_t first_bucket, uint32_t max_buckets, void* entries, uint64_t entries_cap,
+                                uint32_t* counts, uint32_t* n_buckets, uint64_t* n_entries);
+int         kgx_dpt_export_end(kgx_dpt* t);
+int         kgx_dpt_load(kgx_dpt* t, const uint32_t* h, const void* entries32, uint64_t n);
+
 /* --- device-side unit-test / microbenchmark hooks (kgx_field.cuh, kgx_modinv.h) --- */
 /* op: 0 = mul, 1 = sqr, 2 = sub, 3 = inv.  a, b, out: n x 4 limbs on the HOST. */
 int kgx_test_field(int dev, int op, int n, const uint64_t* a, const uint64_t* b, uint64_t* out);

@@ -79,6 +79,16 @@ int kgi_load_work_ex(kgi_table* t, const char* path, uint32_t* dp_bits, uint64_t
                      uint64_t keyx[4], uint64_t keyy[4], uint64_t* total_count, double* total_time,
                      uint64_t* n_walks, uint64_t* walk_offset);
 
+/* Bulk paths in work-file order (bucket h ascending, then x ascending as (x[1], x[0])), for the device table
+ * (include/kgx.h kgx_dpt_*): entries32 = n x 32-byte {x[2], d[2]} entries, h = their buckets.
+ *   kgi_fill_sorted   appends n entries, possibly in several chunks after kgi_reset: O(n), no search.  Each bucket's
+ *                     cap becomes what sequential kgi_add calls of the same entries would record when none is rejected.
+ *                     Returns 0, or -1 (table unchanged) when an h >= 2^18, h decreases inside the chunk or x does not
+ *                     ascend inside a bucket.
+ *   kgi_export_sorted writes entries [first, first + n) of the table in that order; returns how many it wrote. */
+int      kgi_fill_sorted(kgi_table* t, const uint32_t* h, const void* entries32, uint64_t n);
+uint64_t kgi_export_sorted(kgi_table* t, uint64_t first, uint64_t n, uint32_t* h, void* entries32);
+
 #ifdef __cplusplus
 }
 #endif

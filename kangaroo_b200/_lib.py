@@ -56,7 +56,23 @@ _SIGS = {
     "kgx_set_jumps_per_launch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "kgx_kernel_launches": (ctypes.c_uint64, [ctypes.c_void_p]),
     "kgx_debug_prof": (ctypes.c_int, [ctypes.c_void_p, _u64p]),
-    "kgx_test_field": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int, _u64p, _u64p, _u64p]),
+    "kgx_dpt_create": (ctypes.c_void_p, [ctypes.c_int, ctypes.c_uint64, ctypes.c_uint32]),
+    "kgx_dpt_destroy": (None, [ctypes.c_void_p]),
+    "kgx_dpt_last_error": (ctypes.c_char_p, [ctypes.c_void_p]),
+    "kgx_dpt_memory_bytes": (ctypes.c_uint64, [ctypes.c_uint64]),
+    "kgx_dpt_max_capacity": (ctypes.c_uint64, []),
+    "kgx_dpt_capacity": (ctypes.c_uint64, [ctypes.c_void_p]),
+    "kgx_dpt_insert": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.POINTER(ctypes.c_uint32), ctypes.c_uint32,
+                                      ctypes.c_void_p]),
+    "kgx_dpt_events": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.POINTER(ctypes.c_uint32), _u64p]),
+    "kgx_dpt_pending": (ctypes.c_int, [ctypes.c_void_p]),
+    "kgx_dpt_count": (ctypes.c_int, [ctypes.c_void_p, _u64p]),
+    "kgx_dpt_export_begin": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p]),
+    "kgx_dpt_export_read": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_uint64,
+                                           ctypes.c_void_p, ctypes.POINTER(ctypes.c_uint32), _u64p]),
+    "kgx_dpt_export_end": (ctypes.c_int, [ctypes.c_void_p]),
+    "kgx_dpt_load": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64]),
+    "kgx_test_field":(ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int, _u64p, _u64p, _u64p]),
     "kgx_bench_raw": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_float),
                                      ctypes.POINTER(ctypes.c_double)]),
 }

@@ -6,6 +6,8 @@
 // transposes, double-buffered DP slabs so the readback of launch i overlaps launch i+1, CUDA-event timing of
 // every launch.  No CPU fallback exists: every entry point fails when CUDA does.
 #include <cuda_runtime.h>
+#include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
@@ -14,6 +16,7 @@
 #include "kgx_kernel.cuh"
 #include "kgx_herd.cuh"
 #include "kgx_walks.cuh"
+#include "kgx_dptable.cuh"
 
 using namespace kgx;
 
@@ -659,6 +662,293 @@ int kgx_bench_raw(int dev, int kind, int iters, float* ms, double* ops) {
   double per_thread = kind == 0 ? 8.0 * iters : (kind == 3 ? 1.0 * iters : 2.0 * iters);
   *ops = per_thread * (double)blocks * threads;
   cudaFree(sink); cudaEventDestroy(a); cudaEventDestroy(b);
+  return 0;
+}
+
+}  // extern "C"
+
+// ---- device DP table (kgx_dptable.cuh; C ABI include/kgx.h kgx_dpt_*) ----
+namespace {
+constexpr double DPT_LOAD = 0.7;                      // entries per slot at capacity (KGX_DPT_LOAD)
+constexpr uint64_t DPT_TAIL = 1 << 16;                // slots past the last bucket for the last buckets' probes
+constexpr uint32_t DPT_MAX_S = 9000;                  // slots per bucket: keeps a bucket's export sort inside dpt::MAXB
+constexpr uint64_t DPT_SCRATCH = 1 << 22;             // entries of one export / bulk-load chunk (128 MiB)
+constexpr uint32_t DPT_CHUNK_BUCKETS = 4096;          // buckets counted per export read
+constexpr int DPT_RING = 2;                           // inserts whose events have not been collected yet
+
+uint32_t dpt_slots_per_bucket(uint64_t capacity) {
+  const double s = std::ceil((double)capacity / DPT_LOAD / (double)dpt::HASH_SIZE);
+  return s < 1 ? 1u : (s > 4e9 ? 0xFFFFFFFFu : (uint32_t)s);
+}
+uint64_t dpt_table_bytes(uint32_t S) { return ((uint64_t)dpt::HASH_SIZE * S + DPT_TAIL) * 40; }
+char g_dpt_err[256] = "";
+}  // namespace
+
+struct kgx_dpt {
+  int dev = 0;
+  uint64_t capacity = 0;
+  dpt::Table tab{};
+  uint32_t epoch = 0, evCap = 0;
+  cudaStream_t stream = nullptr, expStream = nullptr;
+  // inserts: batch scratch (grown to the largest batch) and a ring of event buffers, device + pinned host
+  uint32_t batchCap = 0;
+  uint32_t* L = nullptr; uint32_t* head = nullptr; unsigned long long* res = nullptr;
+  uint8_t* evDev[DPT_RING] = {nullptr, nullptr};
+  uint8_t* evHost[DPT_RING] = {nullptr, nullptr};
+  cudaEvent_t evDone[DPT_RING] = {nullptr, nullptr};
+  int ringHead = 0, pending = 0;
+  // export / bulk load
+  ulonglong2* scratch = nullptr;
+  uint32_t* dH = nullptr;                             // bulk load: buckets of a chunk
+  uint32_t* dCounts = nullptr; unsigned long long* dOff = nullptr;
+  uint32_t* hCounts = nullptr; unsigned long long* hOff = nullptr;
+  dpt::EvHeader* dHdr = nullptr; dpt::EvHeader* hHdr = nullptr;
+  cudaEvent_t evExp = nullptr;
+  bool exporting = false;
+  uint32_t expEpoch = 0;
+  char err[256] = "";
+};
+
+extern "C" {
+
+const char* kgx_dpt_last_error(kgx_dpt* t) { return t ? t->err : g_dpt_err; }
+
+uint64_t kgx_dpt_memory_bytes(uint64_t capacity) {
+  return dpt_table_bytes(dpt_slots_per_bucket(capacity)) + DPT_SCRATCH * 36 + 8;
+}
+
+uint64_t kgx_dpt_max_capacity(void) { return (uint64_t)(DPT_LOAD * DPT_MAX_S * dpt::HASH_SIZE); }
+
+void kgx_dpt_destroy(kgx_dpt* t) {
+  if (!t) return;
+  cudaSetDevice(t->dev);
+  if (t->stream) cudaStreamSynchronize(t->stream);
+  if (t->expStream) cudaStreamSynchronize(t->expStream);
+  for (int i = 0; i < DPT_RING; i++) {
+    if (t->evDone[i]) { cudaEventSynchronize(t->evDone[i]); cudaEventDestroy(t->evDone[i]); }
+    cudaFree(t->evDev[i]);
+    if (t->evHost[i]) cudaFreeHost(t->evHost[i]);
+  }
+  cudaFree(t->tab.meta); cudaFree(t->tab.ent); cudaFree(t->tab.count);
+  cudaFree(t->L); cudaFree(t->head); cudaFree(t->res);
+  cudaFree(t->scratch); cudaFree(t->dH); cudaFree(t->dCounts); cudaFree(t->dOff); cudaFree(t->dHdr);
+  if (t->hCounts) cudaFreeHost(t->hCounts);
+  if (t->hOff) cudaFreeHost(t->hOff);
+  if (t->hHdr) cudaFreeHost(t->hHdr);
+  if (t->evExp) cudaEventDestroy(t->evExp);
+  if (t->stream) cudaStreamDestroy(t->stream);
+  if (t->expStream) cudaStreamDestroy(t->expStream);
+  delete t;
+}
+
+kgx_dpt* kgx_dpt_create(int dev, uint64_t capacity, uint32_t max_events) {
+  kgx_dpt* t = new kgx_dpt();
+  auto fail = [&](const char* what, cudaError_t s) -> kgx_dpt* {
+    snprintf(g_dpt_err, sizeof g_dpt_err, "kgx_dpt_create: %s: %s", what, cudaGetErrorString(s));
+    cudaGetLastError();
+    kgx_dpt_destroy(t);
+    return nullptr;
+  };
+  if (capacity == 0 || capacity > kgx_dpt_max_capacity() || max_events == 0) {
+    snprintf(g_dpt_err, sizeof g_dpt_err, "kgx_dpt_create: capacity must be in [1, %llu] and max_events > 0",
+             (unsigned long long)kgx_dpt_max_capacity());
+    delete t; return nullptr;
+  }
+  cudaError_t s;
+  if ((s = cudaSetDevice(dev)) != cudaSuccess) return fail("cudaSetDevice", s);
+  t->dev = dev; t->capacity = capacity; t->evCap = max_events;
+  t->tab.S = dpt_slots_per_bucket(capacity);
+  t->tab.nslots = (uint64_t)dpt::HASH_SIZE * t->tab.S + DPT_TAIL;
+  if ((s = cudaStreamCreateWithFlags(&t->stream, cudaStreamNonBlocking)) != cudaSuccess) return fail("cudaStreamCreate", s);
+  if ((s = cudaStreamCreateWithFlags(&t->expStream, cudaStreamNonBlocking)) != cudaSuccess) return fail("cudaStreamCreate", s);
+  if ((s = cudaMalloc(&t->tab.meta, t->tab.nslots * 8)) != cudaSuccess) return fail("cudaMalloc(meta)", s);
+  if ((s = cudaMalloc(&t->tab.ent, t->tab.nslots * 32)) != cudaSuccess) return fail("cudaMalloc(entries)", s);
+  if ((s = cudaMalloc(&t->tab.count, 8)) != cudaSuccess) return fail("cudaMalloc(count)", s);
+  if ((s = cudaMemsetAsync(t->tab.meta, 0, t->tab.nslots * 8, t->stream)) != cudaSuccess) return fail("cudaMemset(meta)", s);
+  if ((s = cudaMemsetAsync(t->tab.count, 0, 8, t->stream)) != cudaSuccess) return fail("cudaMemset(count)", s);
+  const size_t evBytes = sizeof(dpt::EvHeader) + (size_t)max_events * sizeof(dpt::Event);
+  for (int i = 0; i < DPT_RING; i++) {
+    if ((s = cudaMalloc(&t->evDev[i], evBytes)) != cudaSuccess) return fail("cudaMalloc(events)", s);
+    if ((s = cudaHostAlloc(&t->evHost[i], evBytes, cudaHostAllocDefault)) != cudaSuccess) return fail("cudaHostAlloc(events)", s);
+    if ((s = cudaEventCreateWithFlags(&t->evDone[i], cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", s);
+  }
+  if ((s = cudaMalloc(&t->scratch, DPT_SCRATCH * 32)) != cudaSuccess) return fail("cudaMalloc(scratch)", s);
+  if ((s = cudaMalloc(&t->dH, DPT_SCRATCH * 4)) != cudaSuccess) return fail("cudaMalloc(scratch)", s);
+  if ((s = cudaMalloc(&t->dCounts, DPT_CHUNK_BUCKETS * 4)) != cudaSuccess) return fail("cudaMalloc(counts)", s);
+  if ((s = cudaMalloc(&t->dOff, DPT_CHUNK_BUCKETS * 8)) != cudaSuccess) return fail("cudaMalloc(offsets)", s);
+  if ((s = cudaMalloc(&t->dHdr, sizeof(dpt::EvHeader))) != cudaSuccess) return fail("cudaMalloc(header)", s);
+  if ((s = cudaHostAlloc(&t->hCounts, DPT_CHUNK_BUCKETS * 4, cudaHostAllocDefault)) != cudaSuccess) return fail("cudaHostAlloc", s);
+  if ((s = cudaHostAlloc(&t->hOff, DPT_CHUNK_BUCKETS * 8, cudaHostAllocDefault)) != cudaSuccess) return fail("cudaHostAlloc", s);
+  if ((s = cudaHostAlloc(&t->hHdr, sizeof(dpt::EvHeader), cudaHostAllocDefault)) != cudaSuccess) return fail("cudaHostAlloc", s);
+  if ((s = cudaEventCreateWithFlags(&t->evExp, cudaEventDisableTiming)) != cudaSuccess) return fail("cudaEventCreate", s);
+  if ((s = cudaFuncSetAttribute(dpt::export_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dpt::SORT_SMEM)) != cudaSuccess)
+    return fail("cudaFuncSetAttribute(export_sort_kernel)", s);
+  if ((s = cudaStreamSynchronize(t->stream)) != cudaSuccess) return fail("sync", s);
+  return t;
+}
+
+uint64_t kgx_dpt_capacity(kgx_dpt* t) { return t->capacity; }
+
+#define CKT(call)                                                                              \
+  do {                                                                                         \
+    cudaError_t _s = (call);                                                                   \
+    if (_s != cudaSuccess) {                                                                   \
+      snprintf(t->err, sizeof(t->err), "%s: %s", #call, cudaGetErrorString(_s));              \
+      return -3;                                                                               \
+    }                                                                                          \
+  } while (0)
+
+static int dpt_grow(kgx_dpt* t, uint32_t n) {
+  if (n <= t->batchCap) return 0;
+  for (int k = 0; k < t->pending; k++) CKT(cudaEventSynchronize(t->evDone[(t->ringHead + k) % DPT_RING]));   // still in use
+  uint32_t cap = t->batchCap ? t->batchCap : (1u << 16);
+  while (cap < n) cap *= 2;
+  cudaFree(t->L); cudaFree(t->head); cudaFree(t->res);
+  t->L = nullptr; t->head = nullptr; t->res = nullptr; t->batchCap = 0;
+  CKT(cudaMalloc(&t->L, (size_t)cap * 2 * 4));
+  CKT(cudaMalloc(&t->head, (size_t)cap * 4));
+  CKT(cudaMalloc(&t->res, (size_t)cap * 8));
+  t->batchCap = cap;
+  return 0;
+}
+
+int kgx_dpt_insert(kgx_dpt* t, const void* recs, uint32_t stride, const uint32_t* counts, uint32_t nranks, void* stream) {
+  CKT(cudaSetDevice(t->dev));
+  if (nranks == 0 || nranks > (uint32_t)dpt::MAX_RANKS) { snprintf(t->err, sizeof t->err, "kgx_dpt_insert: 1..%d ranks", dpt::MAX_RANKS); return -3; }
+  if (t->pending == DPT_RING) { snprintf(t->err, sizeof t->err, "kgx_dpt_insert: %d inserts pending, collect their events first", DPT_RING); return -3; }
+  dpt::Batch b;
+  b.base = static_cast<const uint32_t*>(recs); b.stride = stride; b.nranks = nranks;
+  uint64_t n = 0;
+  for (uint32_t r = 0; r < nranks; r++) {
+    if (nranks > 1 && counts[r] > stride) { snprintf(t->err, sizeof t->err, "kgx_dpt_insert: rank %u: %u records, stride %u", r, counts[r], stride); return -3; }
+    b.prefix[r] = (uint32_t)n; n += counts[r];
+  }
+  b.prefix[nranks] = (uint32_t)n;
+  if (n >= (1u << 31)) { snprintf(t->err, sizeof t->err, "kgx_dpt_insert: batch too large"); return -3; }
+  if (int rc = dpt_grow(t, (uint32_t)n)) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int slot = (t->ringHead + t->pending) % DPT_RING;
+  dpt::EvHeader* hdr = reinterpret_cast<dpt::EvHeader*>(t->evDev[slot]);
+  dpt::Event* ev = reinterpret_cast<dpt::Event*>(t->evDev[slot] + sizeof(dpt::EvHeader));
+  const uint32_t epoch = ++t->epoch;
+  CKT(cudaMemsetAsync(hdr, 0, sizeof *hdr, st));
+  if (n) {
+    uint32_t lsize = 1;
+    while (lsize < 2 * n) lsize <<= 1;
+    const uint32_t blocks = (uint32_t)((n + 255) / 256);
+    CKT(cudaMemsetAsync(t->L, 0xFF, (size_t)lsize * 4, st));
+    dpt::dedup_kernel<<<blocks, 256, 0, st>>>(b, (uint32_t)n, t->L, lsize - 1, hdr);
+    dpt::head_kernel<<<blocks, 256, 0, st>>>(b, (uint32_t)n, t->L, lsize - 1, t->tab, epoch, t->head, t->res, hdr);
+    dpt::event_kernel<<<blocks, 256, 0, st>>>(b, (uint32_t)n, t->tab, t->head, t->res, hdr, ev, t->evCap);
+  }
+  dpt::snapshot_count_kernel<<<1, 1, 0, st>>>(t->tab.count, hdr);
+  CKT(cudaGetLastError());
+  CKT(cudaMemcpyAsync(t->evHost[slot], t->evDev[slot], sizeof(dpt::EvHeader) + (size_t)t->evCap * sizeof(dpt::Event),
+                      cudaMemcpyDeviceToHost, st));
+  CKT(cudaEventRecord(t->evDone[slot], st));
+  t->pending++;
+  return 0;
+}
+
+int kgx_dpt_events(kgx_dpt* t, void* out, uint32_t cap, uint32_t* n_ev, uint64_t* entries) {
+  CKT(cudaSetDevice(t->dev));
+  *n_ev = 0;
+  if (t->pending == 0) { snprintf(t->err, sizeof t->err, "kgx_dpt_events: no insert pending"); return -3; }
+  const int slot = t->ringHead;
+  CKT(cudaEventSynchronize(t->evDone[slot]));
+  t->ringHead = (t->ringHead + 1) % DPT_RING;
+  t->pending--;
+  const dpt::EvHeader* hdr = reinterpret_cast<const dpt::EvHeader*>(t->evHost[slot]);
+  const uint32_t k = std::min(std::min(hdr->count, cap), t->evCap);
+  memcpy(out, t->evHost[slot] + sizeof(dpt::EvHeader), (size_t)k * sizeof(dpt::Event));
+  *n_ev = hdr->count;
+  if (entries) *entries = hdr->entries;
+  if (hdr->flags & dpt::FLAG_OVERFLOW) { snprintf(t->err, sizeof t->err, "kgx_dpt_events: a probe ran past the table's last slot"); return -2; }
+  return (hdr->flags & dpt::FLAG_BAD) ? -1 : 0;
+}
+
+int kgx_dpt_pending(kgx_dpt* t) { return t->pending; }
+
+int kgx_dpt_count(kgx_dpt* t, uint64_t* entries) {
+  CKT(cudaSetDevice(t->dev));
+  for (int k = 0; k < t->pending; k++) CKT(cudaEventSynchronize(t->evDone[(t->ringHead + k) % DPT_RING]));
+  CKT(cudaMemcpyAsync(&t->hHdr->entries, t->tab.count, 8, cudaMemcpyDeviceToHost, t->stream));
+  CKT(cudaStreamSynchronize(t->stream));
+  *entries = t->hHdr->entries;
+  return 0;
+}
+
+int kgx_dpt_export_begin(kgx_dpt* t, void* stream) {
+  CKT(cudaSetDevice(t->dev));
+  if (t->exporting) { snprintf(t->err, sizeof t->err, "kgx_dpt_export_begin: previous export not ended"); return -3; }
+  t->expEpoch = t->epoch;
+  CKT(cudaEventRecord(t->evExp, static_cast<cudaStream_t>(stream)));
+  t->exporting = true;
+  return 0;
+}
+
+int kgx_dpt_export_read(kgx_dpt* t, uint32_t first_bucket, uint32_t max_buckets, void* entries, uint64_t entries_cap,
+                        uint32_t* counts, uint32_t* n_buckets, uint64_t* n_entries) {
+  CKT(cudaSetDevice(t->dev));
+  *n_buckets = 0; *n_entries = 0;
+  if (!t->exporting) { snprintf(t->err, sizeof t->err, "kgx_dpt_export_read: no export begun"); return -3; }
+  if (first_bucket >= dpt::HASH_SIZE || max_buckets == 0) return 0;
+  const uint32_t nb = std::min(std::min(max_buckets, dpt::HASH_SIZE - first_bucket), DPT_CHUNK_BUCKETS);
+  CKT(cudaStreamWaitEvent(t->expStream, t->evExp, 0));
+  dpt::export_count_kernel<<<nb, 256, 0, t->expStream>>>(t->tab, first_bucket, t->expEpoch, t->dCounts);
+  CKT(cudaGetLastError());
+  CKT(cudaMemcpyAsync(t->hCounts, t->dCounts, (size_t)nb * 4, cudaMemcpyDeviceToHost, t->expStream));
+  CKT(cudaStreamSynchronize(t->expStream));
+  const uint64_t lim = std::min<uint64_t>(entries_cap, DPT_SCRATCH);
+  uint64_t total = 0;
+  uint32_t k = 0;
+  for (; k < nb; k++) {
+    const uint32_t c = t->hCounts[k];
+    if (c > (uint32_t)dpt::MAXB) {
+      snprintf(t->err, sizeof t->err, "kgx_dpt_export_read: bucket %u holds %u entries, more than %d", first_bucket + k, c, dpt::MAXB);
+      return -3;
+    }
+    if (total + c > lim) break;
+    t->hOff[k] = total;
+    total += c;
+  }
+  if (k == 0) { snprintf(t->err, sizeof t->err, "kgx_dpt_export_read: room for %llu entries, bucket %u holds %u",
+                         (unsigned long long)entries_cap, first_bucket, t->hCounts[0]); return -3; }
+  CKT(cudaMemcpyAsync(t->dOff, t->hOff, (size_t)k * 8, cudaMemcpyHostToDevice, t->expStream));
+  dpt::export_sort_kernel<<<k, dpt::SORT_THREADS, dpt::SORT_SMEM, t->expStream>>>(t->tab, first_bucket, t->expEpoch, t->dOff, t->scratch);
+  CKT(cudaGetLastError());
+  if (total) CKT(cudaMemcpyAsync(entries, t->scratch, total * 32, cudaMemcpyDeviceToHost, t->expStream));
+  CKT(cudaStreamSynchronize(t->expStream));
+  memcpy(counts, t->hCounts, (size_t)k * 4);
+  *n_buckets = k; *n_entries = total;
+  return 0;
+}
+
+int kgx_dpt_export_end(kgx_dpt* t) {
+  CKT(cudaSetDevice(t->dev));
+  if (!t->exporting) return 0;
+  CKT(cudaStreamSynchronize(t->expStream));
+  t->exporting = false;
+  return 0;
+}
+
+int kgx_dpt_load(kgx_dpt* t, const uint32_t* h, const void* entries32, uint64_t n) {
+  CKT(cudaSetDevice(t->dev));
+  if (t->pending || t->exporting) { snprintf(t->err, sizeof t->err, "kgx_dpt_load: inserts or an export pending"); return -3; }
+  const uint32_t epoch = ++t->epoch;
+  CKT(cudaMemsetAsync(t->dHdr, 0, sizeof(dpt::EvHeader), t->stream));
+  const uint8_t* e = static_cast<const uint8_t*>(entries32);
+  for (uint64_t o = 0; o < n; o += DPT_SCRATCH) {
+    const uint64_t k = std::min<uint64_t>(DPT_SCRATCH, n - o);
+    CKT(cudaMemcpyAsync(t->dH, h + o, k * 4, cudaMemcpyHostToDevice, t->stream));
+    CKT(cudaMemcpyAsync(t->scratch, e + o * 32, k * 32, cudaMemcpyHostToDevice, t->stream));
+    dpt::load_kernel<<<(uint32_t)((k + 255) / 256), 256, 0, t->stream>>>(t->dH, t->scratch, k, t->tab, epoch, t->dHdr);
+    CKT(cudaGetLastError());
+  }
+  CKT(cudaMemcpyAsync(t->hHdr, t->dHdr, sizeof(dpt::EvHeader), cudaMemcpyDeviceToHost, t->stream));
+  CKT(cudaStreamSynchronize(t->stream));
+  if (t->hHdr->flags & dpt::FLAG_OVERFLOW) { snprintf(t->err, sizeof t->err, "kgx_dpt_load: a probe ran past the table's last slot"); return -2; }
+  if (t->hHdr->flags & dpt::FLAG_BAD) { snprintf(t->err, sizeof t->err, "kgx_dpt_load: h >= 2^18"); return -1; }
   return 0;
 }
 

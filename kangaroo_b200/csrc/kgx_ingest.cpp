@@ -421,6 +421,48 @@ int kgi_load_work(kgi_table* t, const char* path, uint32_t* dp_bits, uint64_t* t
   return 0;
 }
 
+// The cap sequential bucket_add calls leave on a bucket after k entries, none rejected: 16 from the first add, +4 whenever an
+// add finds size >= cap - 1.
+static uint32_t cap_after(uint64_t k) {
+  if (k == 0) return 0;
+  uint32_t cap = 16;
+  if (k >= 16) cap += 4 * (uint32_t)((k - 16) / 4 + 1);
+  return cap;
+}
+
+int kgi_fill_sorted(kgi_table* t, const uint32_t* h, const void* entries32, uint64_t n) {
+  const Entry* e = static_cast<const Entry*>(entries32);
+  for (uint64_t i = 0; i < n; i++) {               // validate first: a refused chunk leaves the table as it was
+    if (h[i] >= HASH_SIZE || (i && h[i] < h[i - 1])) return -1;
+    const Entry* last = nullptr;
+    if (i && h[i - 1] == h[i]) last = &e[i - 1];
+    else if (!t->buckets[h[i]].items.empty()) last = &t->buckets[h[i]].items.back();
+    if (last && !x_less(*last, e[i].x)) return -1;  // not strictly ascending in x inside the bucket
+  }
+  for (uint64_t i = 0; i < n; i++) {
+    Bucket& b = t->buckets[h[i]];
+    b.items.push_back(e[i]);
+    if (i + 1 == n || h[i + 1] != h[i]) b.cap = cap_after(b.items.size());
+  }
+  return 0;
+}
+
+uint64_t kgi_export_sorted(kgi_table* t, uint64_t first, uint64_t n, uint32_t* h, void* entries32) {
+  Entry* out = static_cast<Entry*>(entries32);
+  uint64_t pos = 0, k = 0;
+  for (uint32_t b = 0; b < HASH_SIZE && k < n; b++) {
+    const std::vector<Entry>& items = t->buckets[b].items;
+    const uint64_t sz = items.size();
+    if (pos + sz <= first) { pos += sz; continue; }
+    for (uint64_t j = first > pos ? first - pos : 0; j < sz && k < n; j++, k++) {
+      h[k] = b;
+      out[k] = items[j];
+    }
+    pos += sz;
+  }
+  return k;
+}
+
 // Kangaroo::LoadWork (Backup.cpp:154-200) plus the walk count that follows the table.  t == NULL reads the header and
 // skips the table (what every rank but the table's owner needs on resume).
 int kgi_load_work_ex(kgi_table* t, const char* path, uint32_t* dp_bits, uint64_t range_start[4], uint64_t range_end[4],

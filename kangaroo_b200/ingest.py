@@ -43,6 +43,8 @@ _SIGS = {
                                            ctypes.c_uint64, ctypes.c_double, ctypes.c_uint64, _u64p]),
     "kgi_load_work_ex": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, ctypes.POINTER(ctypes.c_uint32), _u64p, _u64p, _u64p, _u64p,
                                         _u64p, ctypes.POINTER(ctypes.c_double), _u64p, _u64p]),
+    "kgi_fill_sorted": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64]),
+    "kgi_export_sorted": (ctypes.c_uint64, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p]),
 }
 EXPORTED_SYMBOLS = sorted(_SIGS)
 _lib = None
@@ -188,6 +190,23 @@ class DPTable:
     def load_work_ex(self, path):
         """load_work returning the whole header (WorkInfo)."""
         return read_work_info(path, self)
+
+    def fill_sorted(self, h, entries):
+        """Append entries given in work-file order (kgi_fill_sorted): h uint32 [n], entries uint64 [n, 4] = {x[2], d[2]}."""
+        h = np.ascontiguousarray(h, dtype=np.uint32)
+        e = np.ascontiguousarray(entries, dtype=np.uint64).reshape(-1, 4)
+        assert h.shape[0] == e.shape[0]
+        if self._lib.kgi_fill_sorted(self._h, h.ctypes.data_as(ctypes.c_void_p), e.ctypes.data_as(ctypes.c_void_p), h.shape[0]) != 0:
+            raise RuntimeError("kgi_fill_sorted: entries out of work-file order or h >= 2^18")
+
+    def export_sorted(self, first=0, n=None):
+        """Entries [first, first + n) in work-file order (kgi_export_sorted) -> (h uint32 [k], entries uint64 [k, 4])."""
+        n = len(self) - first if n is None else n
+        h = np.empty(max(n, 0), dtype=np.uint32)
+        e = np.empty((max(n, 0), 4), dtype=np.uint64)
+        k = int(self._lib.kgi_export_sorted(self._h, int(first), max(n, 0), h.ctypes.data_as(ctypes.c_void_p),
+                                            e.ctypes.data_as(ctypes.c_void_p)))
+        return h[:k], e[:k]
 
     def load_work(self, path):
         dp, cnt, tm = ctypes.c_uint32(0), ctypes.c_uint64(0), ctypes.c_double(0)

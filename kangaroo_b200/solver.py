@@ -10,8 +10,10 @@ Per step (= one GPUEngine::Launch on every rank) nothing on the data path is Pyt
   engine      kgx_collect(cap=0, relaunch=1): wait for launch i, start launch i+1, no host copy of records
   device      kgx_convert_dps: HashTable::Convert of launch i's DPs -> 40-byte `DP` records (Kangaroo.h:94-101)
   NCCL        all_gather(count) + gather(records) to rank 0          (dist.DPGather, wire "dp40")
-  rank 0      one D2H copy -> (ingest thread, one step behind, overlapping the next launch) kgi_add: the reference's HashTable,
-              bucket-sharded multi-threaded insert (ingest.DPTable)
+  rank 0      device table (dptable.DeviceDPTable, when it fits rank 0's memory): kgx_dpt_insert of the gathered buffer,
+              stream-ordered, no host copy; its events are collected one step later
+              host table otherwise: one D2H copy -> (ingest thread, one step behind, overlapping the next launch) kgi_add:
+              the reference's HashTable, bucket-sharded multi-threaded insert (ingest.DPTable)
               -> events: KGI_EV_COLLISION -> kgi_resolve (CollisionCheck/CheckKey with the reference's Secp256K1)
                          KGI_EV_RESET     -> (rank, kIdx) sent back to the owner, which re-creates that kangaroo
                                              (Kangaroo.cpp:601-609: CreateHerd(1) + SetKangaroo)
@@ -21,8 +23,10 @@ Checkpoints (kangaroo_b200/checkpoint.py for the file protocol).  The table in a
 launches 1..L, its walks are the herd after launch L on every rank and its count the jumps through launch L:
   step s      rank 0 decides, the control word carries "begin"; every rank calls kgx_walks_begin, which converts the
               herd on the device in stream order behind launch L = s + 1 (in flight) and returns at once
-  step s + 1  launch L's records go to the ingest thread and rank 0 queues a save marker right behind them: the ingest
-              thread writes header + table to F.tmp (the step loop stalls only if this outlasts the next step's insert)
+  step s + 1  launch L's records go to the table and rank 0 queues a save marker right behind them: the ingest thread
+              writes header + table to F.tmp (the step loop stalls only if this outlasts the next step's insert); with the
+              device table the marker is an export stream-ordered behind launch L's insert, which a thread of its own turns
+              into F.tmp (kgi_fill_sorted + kgi_save_work_walks) while later inserts go on
   later       the walk offset goes out in a control word; every rank's writer thread copies its walks out in chunks and
               pwrites them; a MIN all-reduce of the ranks' done flags runs each step until all are written; rank 0 then
               fsyncs and renames F.tmp -> F
@@ -50,6 +54,7 @@ from . import checkpoint as ckpt
 from .engine import GPUEngine, NB_JUMP, NB_RUN, WILD, WALK_SIZE, random_herd_arrays
 from .dist import DPGather, SlabView, DP40_BYTES
 from .ingest import DPTable, EV_RESET, EV_COLLISION, read_work_info
+from . import dptable
 
 ORDER = ec.N
 MAX_RESETS = 255          # per step, carried in the control broadcast
@@ -136,14 +141,19 @@ class Solver:
         self.eng.CreateHerdRaw(sc, d128, self.key)
         self.gather = DPGather(self.eng, self.dist, self.rank, self.world, torch, wire="dp40") if self.world > 1 else None
         self.dps = DPTable(threads=ingest_threads) if self.rank == 0 else None      # rank 0: the reference HashTable
+        self.dev = None                     # rank 0: the device table, when chosen (_choose_table)
+        self.table_kind = "host"
+        self._lost_warned = False
         self.work_file, self.work_interval, self.save_kangaroos = work_file, float(work_interval or 0), bool(save_kangaroos)
         self.jumps0, self.time0 = 0, 0.0
         self.loaded = self.bad = 0
         # Two pinned staging buffers: while the ingest thread inserts step k's records, step k+1's land in the other one.  The
         # NCCL kernels of a step cannot start before the jump launch that occupies every SM has finished, so without this
         # decoupling the CPU insert (3-4 ms at 8 GPUs) sat exposed between two launches: 97 instead of 112 GJump/s.
-        self._hosts = ([torch.empty(self.world * max_found * DP40_BYTES, dtype=torch.uint8).pin_memory() for _ in range(2)]
-                       if self.rank == 0 else None)
+        self._hosts = None                  # allocated on the first host-table step
+        self._max_found = max_found
+        self._dpbuf = None                  # single GPU, device table: this step's records, off the engine's buffer
+        self._ck_table = None               # device table: host table a checkpoint is written from
         self._hidx = 0
         self._work = queue.Queue()          # steps' records (at most two in flight, _staging) and checkpoint markers
         self._done = queue.Queue()
@@ -170,8 +180,46 @@ class Solver:
         if resume:
             self._resume(resume, n)
             self.jumps = self.jumps0
+        self.expected_ops = dptable.compute_expected(self.range_power, n * self.world, dp_bits)[0]
+        self.suggested_dp = dptable.suggested_dp(self.range_power, n * self.world)
+        if self.rank == 0:
+            self._choose_table()
+
+    def _choose_table(self):
+        """rank 0: the device table when 2 E entries (at least 1.5 E) fit 3/4 of the free device memory, E = the expected DP
+        count plus the resumed entries; KGX_DPTABLE / KGX_DPTABLE_CAP pin the choice"""
+        loaded = len(self.dps)
+        self.expected_dps = self.expected_ops / 2.0 ** self.dp_bits + loaded
+        free = self.torch.cuda.mem_get_info(self.local)[0]
+        kind, cap = dptable.choose_from_env(self.expected_dps, free)
+        if kind == "device" and loaded > cap:
+            kind = "host"
+        if kind == "device":
+            self.dev = dptable.DeviceDPTable(self.local, cap)
+            if loaded:
+                self.dev.load_from_host(self.dps)
+                self.dps.reset()
+        self.table_kind = kind
+
+    def table_len(self):
+        return self.dev.entries if self.dev is not None else len(self.dps)
+
+    def table_desc(self):
+        if self.dev is None:
+            return "host (%d ingest threads)" % self.dps.threads
+        return "device (%d entries, %.1f GB)" % (self.dev.capacity, self.dev.memory() / 1e9)
 
     # -- rank 0: ingest -------------------------------------------------------------------------------------------
+    def _events(self, events, found, resets):
+        for kind, rk, kidx, d_old, d_new in events:
+            if kind == EV_COLLISION and found is None:
+                found = self.dps.resolve(d_old, d_new, self.key, self.start)     # Kangaroo.cpp:255-302
+                if found is None:
+                    resets.append((rk, kidx))                                    # "unexpected wrong collision, reset kangaroo"
+            elif kind == EV_RESET:
+                resets.append((rk, kidx))
+        return found
+
     def _ingest(self, segments):
         """segments: list of (rank, uint8 numpy view of that rank's 40-byte records).  Returns (key or None, resets)."""
         found, resets = None, []
@@ -179,13 +227,7 @@ class Solver:
         for r, buf in segments:
             if buf.size == 0:
                 continue
-            for kind, rk, kidx, d_old, d_new in self.dps.add_dp40(buf, r):
-                if kind == EV_COLLISION and found is None:
-                    found = self.dps.resolve(d_old, d_new, self.key, self.start)     # Kangaroo.cpp:255-302
-                    if found is None:
-                        resets.append((rk, kidx))                                    # "unexpected wrong collision, reset kangaroo"
-                elif kind == EV_RESET:
-                    resets.append((rk, kidx))
+            found = self._events(self.dps.add_dp40(buf, r), found, resets)
         self.t_ingest += time.perf_counter() - t0
         return found, resets
 
@@ -224,6 +266,8 @@ class Solver:
             self._take(block=True)
         if t0 is not None:
             self.t_stall += time.perf_counter() - t0
+        if self._hosts is None:
+            self._hosts = [self.torch.empty(self.world * self._max_found * DP40_BYTES, dtype=self.torch.uint8).pin_memory() for _ in range(2)]
         host = self._hosts[self._hidx]
         self._hidx ^= 1
         return host
@@ -235,8 +279,55 @@ class Solver:
             self._acc_found = f
         self._acc_resets += r
 
+    def _take_dev(self):
+        """events of the oldest insert queued on the device table"""
+        t0 = time.perf_counter()
+        resets = []
+        f = self._events(self.dev.events(), None, resets)
+        self.t_ingest += time.perf_counter() - t0
+        if self._acc_found is None:
+            self._acc_found = f
+        self._acc_resets += resets
+
+    def _dev_insert(self, ptr, counts, stride):
+        """rank 0: one step's records (device memory) into the device table; False when they would take it past its
+        capacity (the caller then migrates and uses the host table)"""
+        n = sum(counts)
+        if not self.dev.fits(n):
+            while self.dev.pending:                                     # the exact count, then decide
+                self._take_dev()
+            if not self.dev.fits(n):
+                return False
+        while self.dev.pending >= 2:
+            self._take_dev()
+        t0 = time.perf_counter()
+        self.dev.insert(ptr, counts, stride, self.torch.cuda.current_stream().cuda_stream)
+        self.t_ingest += time.perf_counter() - t0
+        return True
+
+    def _migrate(self):
+        """rank 0: the device table is full -- move its content to the host table once and go on there"""
+        t0 = time.perf_counter()
+        ck = self._ck
+        if ck is not None and ck.phase == "table" and getattr(ck, "thread", None) is not None:
+            ck.thread.join()                                            # its export reads the device table
+        while self.dev.pending:
+            self._take_dev()
+        n = self.dev.entries
+        self.dev.to_host(self.dps, self.torch.cuda.current_stream().cuda_stream)
+        cap = self.dev.capacity
+        self.dev.close()
+        self.dev = None
+        self.table_kind = "host"
+        self.t_stall += time.perf_counter() - t0
+        print("DP table: the device table is full (%d of %d entries), moved to the host table in %.2f s; the run goes on there" %
+              (n, cap, time.perf_counter() - t0), flush=True)
+
     def _harvest(self, wait_all=False):
         """results of the inserts finished so far -> (key or None, resets)"""
+        if self.dev is not None:
+            while self.dev.pending > (0 if wait_all else 1):            # one step behind: the newest insert may still run
+                self._take_dev()
         while self._pending and (wait_all or not self._done.empty()):
             self._take(block=True)
         found, resets = self._acc_found, self._acc_resets
@@ -264,11 +355,19 @@ class Solver:
         torch = self.torch
         n_found = self.eng.collect_count(relaunch=relaunch)              # launch i done, launch i+1 running
         cnt = min(n_found, self.eng.maxFound)
+        if n_found > cnt and not self._lost_warned:                       # GPUEngine.cu:641-648
+            print("\nWarning, %d items lost (rank %d)\nHint: Search with less threads (-g) or increse dp (-d)" %
+                  (n_found - cnt, self.rank), flush=True)
+            self._lost_warned = True
         self.jumps += self.eng.nbKangaroo * NB_RUN * self.world
         found, resets = None, []
         if self.gather is not None:
             res = self.gather.step_flat(cnt)                                # rank 0: (counts, cap, device tensor [world*cap*40])
-            if self.rank == 0:
+            if self.rank == 0 and self.dev is not None and self._dev_insert(res[2].data_ptr(), res[0], res[1]):
+                pass
+            elif self.rank == 0:
+                if self.dev is not None:
+                    self._migrate()
                 counts, cap, flat = res
                 nbytes = self.world * cap * DP40_BYTES
                 host = self._staging()
@@ -280,6 +379,19 @@ class Solver:
             if cnt:
                 ptr = self.eng.convert_dps_device_ptr()
                 dev = torch.as_tensor(SlabView(ptr + 4, cnt * DP40_BYTES), device="cuda")
+                if self.dev is not None:
+                    # the engine rewrites its buffer at the next step: the insert reads a copy, ordered before it on this stream
+                    if self._dpbuf is None:
+                        self._dpbuf = torch.empty(self._max_found * DP40_BYTES, dtype=torch.uint8, device="cuda")
+                    self._dpbuf[:cnt * DP40_BYTES].copy_(dev)
+                    ev = torch.cuda.Event()
+                    ev.record()
+                    if self._dev_insert(self._dpbuf.data_ptr(), [cnt], 0):
+                        ev.synchronize()
+                        cnt = 0
+                    else:
+                        self._migrate()
+            if cnt:
                 host = self._staging()
                 host[:cnt * DP40_BYTES].copy_(dev, non_blocking=True)
                 torch.cuda.current_stream().synchronize()
@@ -337,7 +449,28 @@ class Solver:
         ck.count = self.jumps
         ck.time = self.time0 + (time.time() - self._t_run)
         ck.phase = "table"
-        self._work.put(ck)
+        if self.dev is not None:
+            self.dev.export_begin(self.torch.cuda.current_stream().cuda_stream)   # behind launch L's insert
+            ck.thread = threading.Thread(target=self._write_table_dev, args=(ck,), daemon=True)
+            ck.thread.start()
+        else:
+            self._work.put(ck)
+
+    def _write_table_dev(self, ck):
+        """thread of its own, device table: the export of launches 1..L -> a host table in work-file order -> F.tmp"""
+        try:
+            if self._ck_table is None:
+                self._ck_table = DPTable(threads=1)
+            self.dev.export_to_host(self._ck_table)
+            walks = self.eng.nbKangaroo * self.world if self.save_kangaroos else 0
+            off = self._ck_table.save_work_walks(ckpt.tmp_path(ck.path), self.dp_bits, self.start, self.end, self.pub,
+                                                 total_count=ck.count, total_time=ck.time, total_walks=walks)
+            ck.result.put(off)
+        except BaseException as e:
+            ck.result.put(e)
+        finally:
+            if self._ck_table is not None:
+                self._ck_table.reset()                                  # the host copy is not kept between checkpoints
 
     def _ck_offset(self, block):
         """rank 0: the walk offset once the ingest thread wrote header and table (0 while pending, -1 on failure)"""
@@ -409,6 +542,8 @@ class Solver:
     def _ck_release(self, ck):
         """this rank's side of a checkpoint that is over: writer joined, export ended (also when no writer ran, e.g. after a
         failed table write), so the next checkpoint can begin"""
+        if getattr(ck, "thread", None) is not None:
+            ck.thread.join()
         if ck.writer is not None:
             ck.writer.join()
             if ck.writer.error is not None:
@@ -519,7 +654,7 @@ class Solver:
             if verbose and self.rank == 0 and (s % 64 == 63 or self.stop):
                 dt = time.time() - t0
                 print("[%6.1fs] 2^%.2f jumps  %.0f MJump/s  %d DPs  dead %d  ingest %.1f ms/step" %
-                      (self.time0 + dt, np.log2(max(self.jumps, 1)), (self.jumps - self.jumps0) / dt / 1e6, len(self.dps),
+                      (self.time0 + dt, np.log2(max(self.jumps, 1)), (self.jumps - self.jumps0) / dt / 1e6, self.table_len(),
                        self.same_herd, 1e3 * self.t_ingest / steps), flush=True)
             if self.stop:
                 break
@@ -546,9 +681,16 @@ class Solver:
             self._work.put(None)
             self._thread.join(timeout=10)
             self._thread = None
+        if self.dev is not None:
+            while self.dev.pending:
+                self.dev.events()
+            self.dev.close()
+            self.dev = None
         self.eng.close()
         if self.dps is not None:
             self.dps.close()
+        if self._ck_table is not None:
+            self._ck_table.close()
 
 
 def main(argv=None):
@@ -587,8 +729,10 @@ def main(argv=None):
         s = Solver(start, end, pub, dp, grid, seed=a.seed, ingest_threads=a.ingest_threads, work_file=a.work_file,
                    work_interval=a.work_interval, save_kangaroos=a.save_kangaroos, resume=a.resume or None)
         if s.rank == 0:
-            print("Range width: 2^%d  kangaroos/GPU: %d  GPUs: %d  dp: %d  ingest threads: %d" %
-                  (s.range_power, s.eng.nbKangaroo, s.world, dp, s.dps.threads), flush=True)
+            print("Suggested DP: %d" % s.suggested_dp)
+            print("Expected operations: 2^%.2f" % np.log2(s.expected_ops))
+            print("Range width: 2^%d  kangaroos/GPU: %d  GPUs: %d  dp: %d  DP table: %s" %
+                  (s.range_power, s.eng.nbKangaroo, s.world, dp, s.table_desc()), flush=True)
             if a.resume:
                 print("resume: %s  count 2^%.2f  time %.1f s" % (a.resume, np.log2(max(s.jumps0, 1)), s.time0), flush=True)
         key = s.run(a.max_steps)
@@ -596,9 +740,11 @@ def main(argv=None):
             print("Solver rate: %.0f MJump/s steady state (after the first 32 steps), %.0f MJump/s over all %d steps (%.2f s); "
                   "rank-0 ingest %.2f ms/step; %d DPs; %d dead kangaroos re-created" %
                   (s.steady_rate / 1e6, (s.jumps - s.jumps0) / s.elapsed / 1e6, s.steps, s.elapsed, 1e3 * s.t_ingest / max(s.steps, 1),
-                   len(s.dps), s.same_herd))
+                   s.table_len(), s.same_herd))
             print("Total count: %d jumps (2^%.2f)" % (s.jumps, np.log2(max(s.jumps, 1))))
             if a.save_work:
+                if s.dev is not None:
+                    s.dev.to_host(s.dps, s.torch.cuda.current_stream().cuda_stream)
                 s.dps.save_work(a.save_work, dp, start, end, pub, total_count=s.jumps, total_time=s.time0 + s.elapsed)
                 print("work file written: %s" % a.save_work)
             if key is not None and ec.mul(key) == pub:
